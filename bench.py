@@ -18,6 +18,8 @@ merge kernel -> matchNNR acceptance.  pairs/step = kf_batch * 800 * 16 M (unique
              box's host cores, on a bounded sample of the same workload
 
 `--impl reference` runs only the CPU arm (rank 0) and prints the same JSON shape.
+`--dump-outputs DIR` writes the match vector and count of the last timed step (rank 0) as DIR/m12.npy and
+DIR/count.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -62,7 +64,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the per-frame / replay side metrics")
     ap.add_argument("--no-verify", action="store_true", help="skip the untimed verification step / multi-GPU check")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (match vector and accepted "
+                         "count, float64) as DIR/<name>.npy; the inputs depend only on the arguments")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200): the reference arm sizes its sample by timing")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -303,6 +313,14 @@ def dist_check(rank: int, world: int, local_rank: int, dev) -> dict:
     return info
 
 
+def dump_outputs(out_dir: str, count, m12) -> None:
+    """What ShardedDescriptorDB.match_nnr returned in the last timed step: the accepted count and the match vector
+    (database row per query, -1 where rejected), both as float64 (row indices < 2^53 stay exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "count.npy"), count.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "m12.npy"), m12.cpu().numpy().astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 def run_b200(args):
     import torch
@@ -400,6 +418,8 @@ def run_b200(args):
     slice_ms, slice_n = ctx.read_profile()
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     n_matches = int(last[0].item())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, *last)
 
     # ---- timed: end to end (host query batch in pinned memory -> host match vector) ------------
     barrier()

@@ -34,9 +34,15 @@ def test_reference_arm_line():
 
 
 @pytest.mark.gpu
-def test_b200_arm_line():
-    """`bench.py` on the GPU (short: no side metrics, no CPU baseline): roofline, e2e, clocks and launch count."""
-    d = run_bench("--steps", "3", "--warmup", "3", "--no-extras", "--no-cpu-baseline")
+def test_b200_arm_line(tmp_path):
+    """`bench.py` on the GPU (short: no side metrics, no CPU baseline): roofline, e2e, clocks and launch count, and the
+    outputs of the last timed step written by --dump-outputs."""
+    import numpy as np
+    d = run_bench("--steps", "3", "--warmup", "3", "--no-extras", "--no-cpu-baseline", "--dump-outputs", str(tmp_path))
+    m12, count = np.load(tmp_path / "m12.npy"), np.load(tmp_path / "count.npy")
+    assert m12.dtype == np.float64 and m12.shape == (6400,) and count.dtype == np.float64 and count.shape == (1,)
+    assert int(count[0]) == d["matches_last_step"] == int((m12 >= 0).sum()) > 0
+    assert (m12 < d["config"]["db_rows"]).all() and (m12 == np.round(m12)).all()
     assert (BASE_KEYS - {"cpu_baseline"}) <= set(d)
     assert d["n_gpus"] == 1 and d["steps"] == 3 and d["warmup"] == 3 and d["value"] > 1e11
     assert d["gpu_launches"] > 0
