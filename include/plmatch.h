@@ -22,6 +22,8 @@
  *   plm_voc_* / plm_bow_*   DBoW2 vocabulary transform + L1 score behind MapHandler::insertKFBowVectorP/L/PL
  *                           src/mapHandler.cpp:3116-3237; 3rdparty/DBoW2/include/DBoW2/TemplatedVocabulary.h:1045-1238,
  *                           3rdparty/DBoW2/src/DBoW2/{BowVector.cpp:31-81, ScoringObject.cpp:25-69, FORB.cpp:78-100}
+ *   plm_loopdb_*            loop-closure keyframe database: insertKFBowVectorP/L/PL and isLoopClosure's matching on
+ *                           device-resident keyframes   src/mapHandler.cpp:3116-3237, 3325-3378
  *   plm_med_desc / plm_dev_med_desc   PLSLAM::MapPoint / MapLine::updateAverageDescDir (the producer of the
  *                           map's med_desc rows)           src/mapFeatures.cpp:51-93, 121-163
  *
@@ -599,6 +601,50 @@ int plm_dev_bow_score(plm_ctx *ctx, const uint32_t *q_ids_dev, const double *q_v
                       const int32_t *q_len_dev, int n_q, int max_q_len, int64_t n_words, const uint32_t *db_ids_dev,
                       const double *db_vals_dev, const int64_t *db_start_dev, const int32_t *db_len_dev, int n_db,
                       double *scores_dev);
+
+/* ---- loop-closure keyframe database (MapHandler::insertKFBowVectorP / L / PL + isLoopClosure) -------------------- */
+/* The keyframes of MapHandler's loop-closure path, resident on the vocabularies' device: each keyframe's left point and
+ * line descriptors and its BowVector(s) are uploaded / computed once, when it is inserted; nothing about an earlier
+ * keyframe crosses PCIe again.  mode 0 = insertKFBowVectorP (voc_l may be NULL), 1 = insertKFBowVectorL (voc_p may be
+ * NULL), 2 = insertKFBowVectorPL (both; they must live on the same device); fixed per database, as one MapHandler uses
+ * one strategy.  The database runs on the context of voc_p (mode 1: voc_l).  kf_capacity = keyframes the arenas are
+ * first sized for (0 = 64); every arena grows geometrically when needed.  One database object may be used by one host
+ * thread at a time. */
+typedef struct plm_loopdb plm_loopdb;
+int plm_loopdb_create(plm_voc *voc_p, plm_voc *voc_l, int mode, int kf_capacity, plm_loopdb **out);
+int plm_loopdb_destroy(plm_loopdb *db);
+/* Inserts keyframe kf_idx (larger than every earlier kf_idx; gaps allowed) and scores it as insertKFBowVector* does
+ * (mapHandler.cpp:3116-3237): conf_row[j] = score(kf_idx, j) for every live keyframe j < kf_idx, and conf_row[kf_idx] =
+ * its self score; every other entry is left untouched.  Scores are bit-identical to plm_bow_transform + plm_bow_score
+ * (a score without common words is -0.0).  pdesc / ldesc: the keyframe's left point / line descriptors (both are kept
+ * for plm_loopdb_match whatever the mode); a set the mode transforms may hold at most 8192 features
+ * (PLM_E_UNSUPPORTED).  blend = {n_pt, std_pt, n_ls, std_ls} of the PL blend for mode 2 (else ignored, may be NULL):
+ *   s = 0.0 + (sp * n_pt + sl * n_ls) / (n_pt + n_ls);  s = s + (sp * std_pt + sl * std_ls) / (std_ls + std_pt)
+ * in fp64, every operation rounded.  Cost per insert, whatever the database size: one host -> device copy (the
+ * descriptors), 2 launches (3 in mode 2), one device -> host copy of the row, one synchronisation.  A failed insert
+ * (argument error, PLM_E_UNSUPPORTED, allocation failure) leaves the database unchanged. */
+int plm_loopdb_insert(plm_loopdb *db, int kf_idx, const uint8_t *pdesc, int n_p, size_t step_p, const uint8_t *ldesc,
+                      int n_l, size_t step_l, const double *blend, double *conf_row);
+/* map_keyframes[kf_idx] = NULL: the keyframe is skipped by every later insert and match (its storage is kept).
+ * PLM_E_INVALID unless kf_idx is a live keyframe of the database. */
+int plm_loopdb_cull(plm_loopdb *db, int kf_idx);
+/* The stored BowVector of live keyframe kf_idx (descDBoW_P for which = 0, descDBoW_L for which = 1; the vocabulary
+ * must be one the mode scores with): *len entries, ascending word id, to ids / vals, which need room for as many entries
+ * as the keyframe's set had features. */
+int plm_loopdb_bow(plm_loopdb *db, int kf_idx, int which, uint32_t *ids, double *vals, int32_t *len);
+/* isLoopClosure's two StVO::match calls (mapHandler.cpp:3325-3378) for n_pairs candidate pairs, from the resident rows:
+ * points of kf0 against points of kf1[k] with nnr_p -> count_pt[k], m12_pt[k * n_p(kf0) ..]; lines with nnr_l ->
+ * count_ls[k], m12_ls[k * n_l(kf0) ..] (either match array may be NULL).  Results equal plm_match's on the same rows,
+ * including a side with 0 or 1 rows: count 0 and every entry -1 (the reference skips an empty side).  Every keyframe
+ * must be live (PLM_E_INVALID otherwise, before any work). */
+int plm_loopdb_match(plm_loopdb *db, int kf0, const int32_t *kf1, int n_pairs, float nnr_p, float nnr_l, int best_lr,
+                     int32_t *count_pt, int32_t *count_ls, int32_t *m12_pt, int32_t *m12_ls);
+/* Keyframes inserted (culled ones included). */
+int64_t plm_loopdb_size(const plm_loopdb *db);
+/* Cumulative bytes copied host -> device / device -> host by inserts and matches (inserts: exactly the descriptor
+ * rows in, the score row out). */
+int64_t plm_loopdb_h2d_bytes(const plm_loopdb *db);
+int64_t plm_loopdb_d2h_bytes(const plm_loopdb *db);
 
 /* Tuning knobs (measurement / A-B tests only; results never depend on them):
  *   "knn_variant"  -1 = automatic (default: 3 for train sets >= 65 536 rows, 5 for short train sides with >= 2^26 pairs,

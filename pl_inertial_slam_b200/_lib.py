@@ -193,6 +193,15 @@ SIGNATURES = {
     "plm_dev_bow_transform": (C.c_int, [vp, vp, C.c_int64, vp, C.c_int, C.c_int, vp, vp, vp]),
     "plm_bow_score": (C.c_int, [vp, vp, f64p, vp, i32p, C.c_int, vp, f64p, vp, i32p, C.c_int, f64p]),
     "plm_dev_bow_score": (C.c_int, [vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int64, vp, vp, vp, vp, C.c_int, vp]),
+    "plm_loopdb_create": (C.c_int, [vp, vp, C.c_int, C.c_int, C.POINTER(vp)]),
+    "plm_loopdb_destroy": (C.c_int, [vp]),
+    "plm_loopdb_insert": (C.c_int, [vp, C.c_int] + _DESC + _DESC + [f64p, f64p]),
+    "plm_loopdb_cull": (C.c_int, [vp, C.c_int]),
+    "plm_loopdb_bow": (C.c_int, [vp, C.c_int, C.c_int, vp, f64p, i32p]),
+    "plm_loopdb_match": (C.c_int, [vp, C.c_int, i32p, C.c_int, C.c_float, C.c_float, C.c_int, i32p, i32p, i32p, i32p]),
+    "plm_loopdb_size": (C.c_int64, [vp]),
+    "plm_loopdb_h2d_bytes": (C.c_int64, [vp]),
+    "plm_loopdb_d2h_bytes": (C.c_int64, [vp]),
     "plm_med_desc": (C.c_int, [vp, u8p, C.c_int64, C.c_size_t, f64p, i32p, C.c_int, i32p, u8p, f64p]),
     "plm_dev_med_desc": (C.c_int, [vp, vp, C.c_int64, vp, vp, C.c_int, vp, vp, vp, vp]),
     "plm_set_option": (C.c_int, [C.c_char_p, C.c_int]),

@@ -17,7 +17,8 @@ from typing import List, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _lib as L
-from .matching import Context
+from .drivers import SlamConfig
+from .matching import Config, Context
 
 TF_IDF, TF, IDF, BINARY = 0, 1, 2, 3   # DBoW2::WeightingType (BowVector.h:38-44)
 L1_NORM = 0                            # DBoW2::ScoringType (BowVector.h:47-55)
@@ -215,3 +216,162 @@ class BowConfusion:
         self.conf_matrix[live, idx] = s
         self.conf_matrix[idx, idx] = blend(np.float64(sp_self), np.float64(sl_self))
         self.map_keyframes[idx] = kf
+
+
+class LoopClosureDB:
+    """The BowConfusion bookkeeping and isLoopClosure's matching over keyframes resident on the device (plm_loopdb_*,
+    include/plmatch.h).  Each keyframe's left point / line descriptors are uploaded once, by its insert; its BowVector(s)
+    are computed into the database's arenas on the device, and every later insert and match reads them there, so the
+    per-insert cost does not grow with the number of earlier keyframes (BowConfusion re-packs and re-uploads all of them
+    on every insert).  Rows of conf_matrix are bit-identical to BowConfusion's for the same insert / cull sequence.
+
+    ``mode``: 0 / "P", 1 / "L" or 2 / "PL" -- the insert strategy, fixed per database (one MapHandler uses one).  The
+    database runs on the vocabularies' context; ``capacity``: keyframes the device arenas are first sized for (0 = a
+    small default; they grow as needed).  One host thread at a time per database."""
+
+    MODES = {"P": 0, "L": 1, "PL": 2}
+
+    def __init__(self, dbow_voc_p: Optional[Vocabulary], dbow_voc_l: Optional[Vocabulary], mode, ctx: Optional[Context] = None,
+                 capacity: int = 0):
+        self.lib = L.load()
+        self.mode = self.MODES[mode] if isinstance(mode, str) else int(mode)
+        self.dbow_voc_p, self.dbow_voc_l = dbow_voc_p, dbow_voc_l
+        first = dbow_voc_l if self.mode == 1 else dbow_voc_p
+        if ctx is not None and first is not None and first.ctx is not ctx:
+            raise ValueError("the database runs on the context of its vocabularies")
+        self.ctx = ctx if ctx is not None else (first.ctx if first is not None else None)
+        self._h = C.c_void_p()
+        L.check(self.lib.plm_loopdb_create(dbow_voc_p._h if dbow_voc_p is not None else None,
+                                           dbow_voc_l._h if dbow_voc_l is not None else None, self.mode, int(capacity),
+                                           C.byref(self._h)), "plm_loopdb_create")
+        self.map_keyframes: List[Optional[KeyFrameBow]] = []
+        self._buf = np.zeros((0, 0), np.float64)   # conf_matrix = _buf[:n, :n]; capacity grows geometrically
+        self._n = 0
+        self._live = np.zeros(0, bool)
+        self._sizes = {}                           # kf_idx -> (point rows, line rows)
+
+    @property
+    def conf_matrix(self) -> np.ndarray:
+        return self._buf[:self._n, :self._n]
+
+    def _grow(self, idx: int):
+        n = idx + 1
+        if n > self._buf.shape[0]:                 # expandGraphs (mapHandler.cpp:874-896) keeps it square
+            cap = max(n, 2 * self._buf.shape[0], 64)
+            m = np.zeros((cap, cap), np.float64)
+            m[:self._n, :self._n] = self.conf_matrix
+            self._buf = m
+            live = np.zeros(cap, bool)
+            live[:len(self._live)] = self._live
+            self._live = live
+        self._n = max(self._n, n)
+        while len(self.map_keyframes) < n:
+            self.map_keyframes.append(None)
+
+    def _insert(self, kf: KeyFrameBow, blend) -> None:
+        idx = int(kf.kf_idx)
+        pd, pp, n_p, sp = L.desc_args(kf.pdesc_l)
+        ld, lp, n_l, sl = L.desc_args(kf.ldesc_l)
+        b = None if blend is None else np.ascontiguousarray(blend, np.float64)
+        n0, k0 = self._n, len(self.map_keyframes)
+        self._grow(idx)
+        row = self._buf[idx]
+        st = self.lib.plm_loopdb_insert(self._h, idx, pp, n_p, sp, lp, n_l, sl, None if b is None else _p(b, L.f64p),
+                                        _p(row, L.f64p))
+        if st != L.PLM_OK:                         # the database is unchanged: so is the matrix
+            self._n = n0
+            del self.map_keyframes[k0:]
+            L.check(st, "plm_loopdb_insert")
+        live = np.flatnonzero(self._live[:idx])
+        self._buf[live, idx] = row[live]
+        self._live[idx] = True
+        self.map_keyframes[idx] = kf
+        self._sizes[idx] = (n_p, n_l)
+
+    def _need(self, mode: int, name: str):
+        if self.mode != mode:
+            raise ValueError(f"{name} called on a database created for mode {self.mode}")
+
+    def insertKFBowVectorP(self, kf: KeyFrameBow) -> None:
+        """mapHandler.cpp:3116-3139."""
+        self._need(0, "insertKFBowVectorP")
+        self._insert(kf, None)
+
+    def insertKFBowVectorL(self, kf: KeyFrameBow) -> None:
+        """mapHandler.cpp:3141-3164."""
+        self._need(1, "insertKFBowVectorL")
+        self._insert(kf, None)
+
+    def insertKFBowVectorPL(self, kf: KeyFrameBow) -> None:
+        """mapHandler.cpp:3166-3237; the dispersion terms are computed on the host as in BowConfusion."""
+        self._need(2, "insertKFBowVectorPL")
+        std_pt = vector_stdv(kf.pt_xy[:, 0]) + vector_stdv(kf.pt_xy[:, 1])
+        std_ls = vector_stdv(kf.ls_mid_xy[:, 0]) + vector_stdv(kf.ls_mid_xy[:, 1])
+        self._insert(kf, [float(len(kf.pt_xy)), std_pt, float(len(kf.ls_mid_xy)), std_ls])
+
+    def cull(self, idx: int) -> None:
+        """map_keyframes[idx] = NULL: skipped by every later insert and match."""
+        L.check(self.lib.plm_loopdb_cull(self._h, int(idx)), "plm_loopdb_cull")
+        self.map_keyframes[idx] = None
+        self._live[idx] = False
+
+    def bow_vector(self, idx: int, which: str = "P") -> BowVector:
+        """descDBoW_P (which = "P") or descDBoW_L ("L") of keyframe idx, read back from the device."""
+        w = {"P": 0, "L": 1}[which] if isinstance(which, str) else int(which)
+        n = self._sizes.get(int(idx), (0, 0))[w]
+        ids, vals, k = np.zeros(max(n, 1), np.uint32), np.zeros(max(n, 1), np.float64), C.c_int32(0)
+        L.check(self.lib.plm_loopdb_bow(self._h, int(idx), w, _p(ids, C.c_void_p), _p(vals, L.f64p), C.byref(k)),
+                "plm_loopdb_bow")
+        return ids[:k.value].copy(), vals[:k.value].copy()
+
+    def match_candidates(self, kf0, kf1_list) -> List[dict]:
+        """isLoopClosure's matching + inlier-ratio gate (mapHandler.cpp:3325-3400) of kf0 against every keyframe of
+        kf1_list (keyframes or indices), from the resident descriptors; the dicts of drivers.loopClosureMatch."""
+        i0 = int(getattr(kf0, "kf_idx", kf0))
+        ks = np.ascontiguousarray([int(getattr(k, "kf_idx", k)) for k in kf1_list], np.int32)
+        n = len(ks)
+        p0, l0 = self._sizes.get(i0, (0, 0))
+        cp, cl = np.zeros(max(n, 1), np.int32), np.zeros(max(n, 1), np.int32)
+        mp, ml = np.zeros((max(n, 1), p0), np.int32), np.zeros((max(n, 1), l0), np.int32)
+        L.check(self.lib.plm_loopdb_match(self._h, i0, _p(ks, L.i32p), n, C.c_float(Config.minRatio12P),
+                                          C.c_float(Config.minRatio12L), int(bool(Config.bestLRMatches)), _p(cp, L.i32p),
+                                          _p(cl, L.i32p), _p(mp, L.i32p), _p(ml, L.i32p)), "plm_loopdb_match")
+        out = []
+        for k in range(n):
+            p1, l1 = self._sizes[int(ks[k])]
+            with_pt, with_ls = bool(p0 and p1), bool(l0 and l1)    # an empty side is not matched (:3333, :3350)
+            common_pt, m_pt = (int(cp[k]), mp[k].copy()) if with_pt else (0, np.zeros(0, np.int32))
+            common_ls, m_ls = (int(cl[k]), ml[k].copy()) if with_ls else (0, np.zeros(0, np.int32))
+            with np.errstate(divide="ignore", invalid="ignore"):
+                r_pt = max(np.float64(100.0 * common_pt) / p0, np.float64(100.0 * common_pt) / p1) if with_pt else 0.0
+                r_ls = max(np.float64(100.0 * common_ls) / l0, np.float64(100.0 * common_ls) / l1) if with_ls else 0.0
+            ok = bool(r_pt > SlamConfig.lcInlierRatio and r_ls > SlamConfig.lcInlierRatio)
+            out.append(dict(common_pt=common_pt, common_ls=common_ls, matches_pt=m_pt, matches_ls=m_ls,
+                            inl_ratio_pt=float(r_pt), inl_ratio_ls=float(r_ls), inl_ratio_condition=ok))
+        return out
+
+    def isLoopClosure(self, kf0, kf1) -> dict:
+        """MapHandler::isLoopClosure's matching and gate for one candidate: drivers.loopClosureMatch's dict."""
+        return self.match_candidates(kf0, [kf1])[0]
+
+    @property
+    def h2d_bytes(self) -> int:
+        return int(self.lib.plm_loopdb_h2d_bytes(self._h))
+
+    @property
+    def d2h_bytes(self) -> int:
+        return int(self.lib.plm_loopdb_d2h_bytes(self._h))
+
+    def __len__(self) -> int:
+        return int(self.lib.plm_loopdb_size(self._h))
+
+    def close(self):
+        if self._h:
+            self.lib.plm_loopdb_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

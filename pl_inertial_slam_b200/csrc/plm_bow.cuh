@@ -69,91 +69,135 @@ struct BowTransformArgs {
 
 inline size_t bow_transform_smem(int cap) { return size_t(cap) * (8 + 8 + 4) + 64; }
 
-// One CTA per descriptor set.
-__global__ void __launch_bounds__(BOW_THREADS) bow_transform_kernel(BowTransformArgs a) {
+// The BowVector of ONE descriptor set (rows lo .. lo + n - 1 of desc, n <= cap), by the whole CTA: written to
+// out_ids / out_vals [out_lo, out_lo + len); returns len.  cap (a power of two) is the shared-memory sort width; the result does
+// not depend on it.  Shared by bow_transform_kernel (many sets) and bow_transform_slots_kernel (the loop-closure
+// database: one set per vocabulary, straight into the database's arenas).
+__device__ __forceinline__ int bow_transform_set(const VocDev &voc, const uint4 *desc, long long lo, int n, int cap,
+                                                 uint32_t *out_ids, double *out_vals, long long out_lo) {
     extern __shared__ __align__(16) unsigned char bow_smem[];
     unsigned long long *keys = reinterpret_cast<unsigned long long *>(bow_smem);    // cap: (word << 32 | leaf), sorted
-    double *vals = reinterpret_cast<double *>(bow_smem + size_t(a.cap) * 8);        // cap: values in word order
-    uint32_t *ids = reinterpret_cast<uint32_t *>(bow_smem + size_t(a.cap) * 16);    // cap
+    double *vals = reinterpret_cast<double *>(bow_smem + size_t(cap) * 8);          // cap: values in word order
+    uint32_t *ids = reinterpret_cast<uint32_t *>(bow_smem + size_t(cap) * 16);      // cap
     __shared__ int s_scan[BOW_THREADS];
     __shared__ double s_norm;
     const int tid = threadIdx.x;
+    // 1. tree descent, one feature per thread
+    for (int f = tid; f < cap; f += BOW_THREADS) {
+        unsigned long long key = KEY64_ABSENT;
+        if (f < n && voc.n_nodes > 1) {
+            const int leaf = bow_descend(voc, load_desc(desc, lo + f));
+            if (__ldg(voc.node_weight + leaf) > 0.0) // stopped words are dropped (:1074)
+                key = make_key64(static_cast<uint32_t>(__ldg(voc.node_word + leaf)), static_cast<uint32_t>(leaf));
+        }
+        keys[f] = key;
+    }
+    __syncthreads();
+    // 2. bitonic sort of the keys (ascending word id == std::map order; absent keys sink to the end)
+    for (int k = 2; k <= cap; k <<= 1) {
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < cap; i += BOW_THREADS) {
+                const int p = i ^ j;
+                if (p > i) {
+                    const unsigned long long x = keys[i], y = keys[p];
+                    const bool up = (i & k) == 0;
+                    if ((x > y) == up) {
+                        keys[i] = y;
+                        keys[p] = x;
+                    }
+                }
+            }
+            __syncthreads();
+        }
+    }
+    // 3. one entry per distinct word: every thread owns a contiguous slice of the sorted keys
+    const int per = (cap + BOW_THREADS - 1) / BOW_THREADS;
+    const int i0 = tid * per, i1 = min(i0 + per, cap);
+    int heads = 0;
+    for (int i = i0; i < i1; ++i) {
+        const unsigned long long k = keys[i];
+        if (k != KEY64_ABSENT && (i == 0 || (keys[i - 1] >> 32) != (k >> 32))) ++heads;
+    }
+    s_scan[tid] = heads;
+    __syncthreads();
+    for (int off = 1; off < BOW_THREADS; off <<= 1) { // inclusive Hillis-Steele scan of the head counts
+        const int v = tid >= off ? s_scan[tid - off] : 0;
+        __syncthreads();
+        s_scan[tid] += v;
+        __syncthreads();
+    }
+    const int len = s_scan[BOW_THREADS - 1];
+    int pos = s_scan[tid] - heads;
+    for (int i = i0; i < i1; ++i) {
+        const unsigned long long k = keys[i];
+        if (k == KEY64_ABSENT || (i > 0 && (keys[i - 1] >> 32) == (k >> 32))) continue;
+        const double w = __ldg(voc.node_weight + static_cast<uint32_t>(k));
+        double v = w; // insert(id, w)
+        if (voc.weighting <= 1) // TF_IDF / TF: addWeight once per further occurrence
+            for (int j = i + 1; j < cap && (keys[j] >> 32) == (k >> 32); ++j) v = __dadd_rn(v, w);
+        ids[pos] = static_cast<uint32_t>(k >> 32);
+        vals[pos] = v;
+        ++pos;
+    }
+    __syncthreads();
+    // 4. BowVector::normalize(L1): sequential sum in word order
+    if (tid == 0) {
+        double norm = 0.0;
+        for (int i = 0; i < len; ++i) norm = __dadd_rn(norm, fabs(vals[i]));
+        s_norm = norm;
+    }
+    __syncthreads();
+    const double norm = s_norm;
+    for (int i = tid; i < len; i += BOW_THREADS) {
+        out_ids[out_lo + i] = ids[i];
+        out_vals[out_lo + i] = norm > 0.0 ? __ddiv_rn(vals[i], norm) : vals[i];
+    }
+    __syncthreads();
+    return len;
+}
+
+// One CTA per descriptor set.
+__global__ void __launch_bounds__(BOW_THREADS) bow_transform_kernel(BowTransformArgs a) {
     for (int s = blockIdx.x; s < a.n_sets; s += gridDim.x) {
         const int lo = __ldg(a.set_start + s);
         const int n = min(max(__ldg(a.set_start + s + 1) - lo, 0), a.cap);
-        // 1. tree descent, one feature per thread
-        for (int f = tid; f < a.cap; f += BOW_THREADS) {
-            unsigned long long key = KEY64_ABSENT;
-            if (f < n && a.voc.n_nodes > 1) {
-                const int leaf = bow_descend(a.voc, load_desc(a.desc, static_cast<long long>(lo) + f));
-                if (__ldg(a.voc.node_weight + leaf) > 0.0) // stopped words are dropped (:1074)
-                    key = make_key64(static_cast<uint32_t>(__ldg(a.voc.node_word + leaf)), static_cast<uint32_t>(leaf));
-            }
-            keys[f] = key;
-        }
-        __syncthreads();
-        // 2. bitonic sort of the keys (ascending word id == std::map order; absent keys sink to the end)
-        for (int k = 2; k <= a.cap; k <<= 1) {
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int i = tid; i < a.cap; i += BOW_THREADS) {
-                    const int p = i ^ j;
-                    if (p > i) {
-                        const unsigned long long x = keys[i], y = keys[p];
-                        const bool up = (i & k) == 0;
-                        if ((x > y) == up) {
-                            keys[i] = y;
-                            keys[p] = x;
-                        }
-                    }
-                }
-                __syncthreads();
-            }
-        }
-        // 3. one entry per distinct word: every thread owns a contiguous slice of the sorted keys
-        const int per = (a.cap + BOW_THREADS - 1) / BOW_THREADS;
-        const int i0 = tid * per, i1 = min(i0 + per, a.cap);
-        int heads = 0;
-        for (int i = i0; i < i1; ++i) {
-            const unsigned long long k = keys[i];
-            if (k != KEY64_ABSENT && (i == 0 || (keys[i - 1] >> 32) != (k >> 32))) ++heads;
-        }
-        s_scan[tid] = heads;
-        __syncthreads();
-        for (int off = 1; off < BOW_THREADS; off <<= 1) { // inclusive Hillis-Steele scan of the head counts
-            const int v = tid >= off ? s_scan[tid - off] : 0;
-            __syncthreads();
-            s_scan[tid] += v;
-            __syncthreads();
-        }
-        const int len = s_scan[BOW_THREADS - 1];
-        int pos = s_scan[tid] - heads;
-        for (int i = i0; i < i1; ++i) {
-            const unsigned long long k = keys[i];
-            if (k == KEY64_ABSENT || (i > 0 && (keys[i - 1] >> 32) == (k >> 32))) continue;
-            const double w = __ldg(a.voc.node_weight + static_cast<uint32_t>(k));
-            double v = w; // insert(id, w)
-            if (a.voc.weighting <= 1) // TF_IDF / TF: addWeight once per further occurrence
-                for (int j = i + 1; j < a.cap && (keys[j] >> 32) == (k >> 32); ++j) v = __dadd_rn(v, w);
-            ids[pos] = static_cast<uint32_t>(k >> 32);
-            vals[pos] = v;
-            ++pos;
-        }
-        __syncthreads();
-        // 4. BowVector::normalize(L1): sequential sum in word order
-        if (tid == 0) {
-            double norm = 0.0;
-            for (int i = 0; i < len; ++i) norm = __dadd_rn(norm, fabs(vals[i]));
-            s_norm = norm;
-        }
-        __syncthreads();
-        const double norm = s_norm;
-        for (int i = tid; i < len; i += BOW_THREADS) {
-            a.bow_ids[lo + i] = ids[i];
-            a.bow_vals[lo + i] = norm > 0.0 ? __ddiv_rn(vals[i], norm) : vals[i];
-        }
-        if (tid == 0) a.bow_len[s] = len;
-        __syncthreads();
+        const int len = bow_transform_set(a.voc, a.desc, lo, n, a.cap, a.bow_ids, a.bow_vals, lo);
+        if (threadIdx.x == 0) a.bow_len[s] = len;
     }
+}
+
+// ---- loop-closure keyframe database (plm_loopdb_*) ----
+// Per vocabulary the database keeps an ids / vals arena and, per keyframe slot, the first entry (start) and the entry
+// count (len) of the slot's BowVector; one live flag per slot is shared by both vocabularies.
+struct LoopVocArgs {
+    VocDev voc;
+    long long desc_lo;   // first row of the new keyframe's set in the descriptor arena
+    int n;               // features in the set
+    int cap;             // power of two >= n (this CTA's sort width)
+    long long entry_lo;  // first entry reserved for the set in the arena (n entries are reserved)
+    uint32_t *ids;       // the vocabulary's arenas and slot tables
+    double *vals;
+    long long *start;
+    int32_t *len;
+};
+
+struct LoopTransformArgs {
+    LoopVocArgs v[2];    // one per vocabulary the database scores with
+    const uint4 *desc;   // the descriptor arena
+    uint8_t *live;       // per slot
+    int slot;            // the new keyframe's slot
+};
+
+// One CTA per vocabulary: the new keyframe's BowVector straight into the arena at its reserved entries, its slot's
+// start / len, and its live flag.
+__global__ void __launch_bounds__(BOW_THREADS) bow_transform_slots_kernel(LoopTransformArgs a) {
+    const LoopVocArgs &v = a.v[blockIdx.x];
+    if (threadIdx.x == 0) {
+        v.start[a.slot] = v.entry_lo;
+        if (blockIdx.x == 0) a.live[a.slot] = 1;
+    }
+    const int len = bow_transform_set(v.voc, a.desc, v.desc_lo, v.n, v.cap, v.ids, v.vals, v.entry_lo);
+    if (threadIdx.x == 0) v.len[a.slot] = len;
 }
 
 struct BowScoreArgs {
@@ -289,13 +333,25 @@ __device__ __forceinline__ uint32_t bow_spread4(uint32_t v) {
 // position among the chunk's candidates comes from one packed warp prefix sum of the eight per-load counts; candidates
 // are written at that position into the warp's pending list and resolved together by bow_flush at the end of the
 // vector (or when 32 are pending).  A chunk with more than 32 candidates takes bow_dense_chunk.
-__global__ void __launch_bounds__(512) bow_score_kernel(BowScoreArgs a) {
+// Shared-memory layout of a scoring CTA and the staging of query q: its values, the hash table word id -> position and
+// the membership bitmap.  The sizes come from the arguments, so CTAs of one launch may score with different vocabularies.
+struct BowScoreSmem {
+    double *qv;
+    uint2 *table;
+    uint32_t *bitmap;
+    long long *pend_all;
+};
+
+__device__ __forceinline__ BowScoreSmem bow_score_stage(const BowScoreArgs &a, int q) {
     extern __shared__ __align__(16) unsigned char bow_smem[];
-    double *qv = reinterpret_cast<double *>(bow_smem);
-    uint2 *table = reinterpret_cast<uint2 *>(bow_smem + size_t(a.q_cap) * 8);
-    uint32_t *bitmap = reinterpret_cast<uint32_t *>(table + a.table_slots);
-    long long *pend_all = reinterpret_cast<long long *>(reinterpret_cast<unsigned char *>(bitmap) + ((size_t(a.bitmap_words + 1) * 4 + 7) & ~size_t(7)));
-    const int q = blockIdx.y;
+    BowScoreSmem s;
+    s.qv = reinterpret_cast<double *>(bow_smem);
+    s.table = reinterpret_cast<uint2 *>(bow_smem + size_t(a.q_cap) * 8);
+    s.bitmap = reinterpret_cast<uint32_t *>(s.table + a.table_slots);
+    s.pend_all = reinterpret_cast<long long *>(reinterpret_cast<unsigned char *>(s.bitmap) + ((size_t(a.bitmap_words + 1) * 4 + 7) & ~size_t(7)));
+    double *qv = s.qv;
+    uint2 *table = s.table;
+    uint32_t *bitmap = s.bitmap;
     const long long qs = __ldg(a.q_start + q);
     const int qn = min(__ldg(a.q_len + q), a.q_cap);
     for (int i = threadIdx.x; i < a.bitmap_words; i += blockDim.x) bitmap[i] = 0u;
@@ -312,11 +368,104 @@ __global__ void __launch_bounds__(512) bow_score_kernel(BowScoreArgs a) {
         table[h].y = static_cast<uint32_t>(i);
     }
     __syncthreads();
+    return s;
+}
+
+// The per-vector loop, by one warp: the L1 sum of the staged query against the database vector at entries
+// [ds, end), before the final -score / 2.
+__device__ __forceinline__ double bow_score_vector(const BowScoreArgs &a, const BowScoreSmem &s, long long ds, long long end) {
+    const double *qv = s.qv;
+    const uint2 *table = s.table;
+    const uint32_t *bitmap = s.bitmap;
     const int lane = threadIdx.x & 31;
-    const int warps = blockDim.x >> 5;
-    long long *pend = pend_all + 32 * (threadIdx.x >> 5);
+    long long *pend = s.pend_all + 32 * (threadIdx.x >> 5);
     const bool vec = (reinterpret_cast<uintptr_t>(a.db_ids) & 15) == 0;
     const uint32_t bwords = static_cast<uint32_t>(a.bitmap_words);
+    double score = 0.0;
+    int n_pend = 0; // warp-uniform
+    // 16-byte groups start at a multiple of 4 entries; the group holding `ds` may begin up to 3 entries early and
+    // the one holding `end - 1` may reach up to 3 entries further -- inside the same 16 aligned bytes as a valid
+    // entry, hence mapped; the validity mask drops them
+    const long long A = vec ? (ds & ~3LL) : ds;
+    for (long long c0 = A; c0 < end; c0 += 1024) {
+        const long long e0 = c0 + 4 * lane; // entry of component 0 of this lane's first load; load i is 128 entries on
+        uint4 r[8];
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            r[i] = make_uint4(0, 0, 0, 0);
+            const long long e = e0 + 128 * i;
+            if (e < end) {
+                if (vec) {
+                    r[i] = __ldg(reinterpret_cast<const uint4 *>(a.db_ids + e));
+                } else { // arena not 16-byte aligned: one id at a time
+                    r[i].x = __ldg(a.db_ids + e);
+                    if (e + 1 < end) r[i].y = __ldg(a.db_ids + e + 1);
+                    if (e + 2 < end) r[i].z = __ldg(a.db_ids + e + 2);
+                    if (e + 3 < end) r[i].w = __ldg(a.db_ids + e + 3);
+                }
+            }
+        }
+        const int left = static_cast<int>(min(end - e0, 4096LL));   // entries from e0 to the end of the vector
+        const int skip = static_cast<int>(min(max(ds - e0, 0LL), 4LL)); // > 0 only in the very first load of the vector
+        uint32_t mb = 0;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            uint32_t nib = bow_maybe(bitmap, bwords, r[i].x) | (bow_maybe(bitmap, bwords, r[i].y) << 1) |
+                           (bow_maybe(bitmap, bwords, r[i].z) << 2) | (bow_maybe(bitmap, bwords, r[i].w) << 3);
+            const int n_valid = min(max(left - 128 * i, 0), 4);
+            nib &= (1u << n_valid) - 1u;
+            if (i == 0) nib &= ~((1u << skip) - 1u);
+            mb |= nib << (4 * i);
+        }
+        if (!__ballot_sync(0xFFFFFFFFu, mb != 0)) continue;
+        // per-load candidate counts of this lane, packed one byte each, and their inclusive prefix over the lanes
+        uint32_t x = mb - ((mb >> 1) & 0x55555555u);
+        x = (x & 0x33333333u) + ((x >> 2) & 0x33333333u); // a popcount per nibble
+        const uint32_t own0 = bow_spread4(x & 0xFFFFu), own1 = bow_spread4(x >> 16);
+        uint32_t in0 = own0, in1 = own1;
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const uint32_t t0 = __shfl_up_sync(0xFFFFFFFFu, in0, off), t1 = __shfl_up_sync(0xFFFFFFFFu, in1, off);
+            if (lane >= off) {
+                in0 += t0; // a byte never exceeds 128 (32 lanes x 4)
+                in1 += t1;
+            }
+        }
+        const uint32_t tot0 = __shfl_sync(0xFFFFFFFFu, in0, 31), tot1 = __shfl_sync(0xFFFFFFFFu, in1, 31);
+        const int sum0 = static_cast<int>(__vsadu4(tot0, 0u)), total = sum0 + static_cast<int>(__vsadu4(tot1, 0u));
+        if (total > 32) {
+            if (n_pend) score = bow_flush(a, qv, table, pend, n_pend, score);
+            n_pend = 0;
+            score = bow_dense_chunk(a, qv, table, bitmap, c0, ds, end, score);
+            continue;
+        }
+        if (n_pend + total > 32) {
+            score = bow_flush(a, qv, table, pend, n_pend, score);
+            n_pend = 0;
+        }
+        // rank of the first candidate of load i of this lane = candidates of the loads before i (all lanes) +
+        // candidates of load i in the lanes below; every byte stays <= 32 here
+        const uint32_t rk0 = tot0 * 0x01010100u + (in0 - own0);
+        const uint32_t rk1 = tot1 * 0x01010100u + static_cast<uint32_t>(sum0) * 0x01010101u + (in1 - own1);
+        uint32_t m = mb;
+        while (m) {
+            const int k = __ffs(m) - 1, i = k >> 2;
+            const uint32_t rk = ((i < 4 ? rk0 : rk1) >> (8 * (i & 3))) & 0xFFu;
+            const uint32_t before = __popc((mb >> (4 * i)) & ((1u << (k & 3)) - 1u));
+            pend[n_pend + rk + before] = e0 + 128 * i + (k & 3);
+            m &= m - 1;
+        }
+        n_pend += total;
+    }
+    if (n_pend) score = bow_flush(a, qv, table, pend, n_pend, score);
+    return score;
+}
+
+__global__ void __launch_bounds__(512) bow_score_kernel(BowScoreArgs a) {
+    const int q = blockIdx.y;
+    const BowScoreSmem s = bow_score_stage(a, q);
+    const int lane = threadIdx.x & 31;
+    const int warps = blockDim.x >> 5;
     const int stride = gridDim.x * warps;
     int j = blockIdx.x * warps + (threadIdx.x >> 5);
     long long nx_ds = 0;
@@ -332,85 +481,45 @@ __global__ void __launch_bounds__(512) bow_score_kernel(BowScoreArgs a) {
             nx_ds = __ldg(a.db_start + j + stride);
             nx_dn = __ldg(a.db_len + j + stride);
         }
-        double score = 0.0;
-        int n_pend = 0; // warp-uniform
-        // 16-byte groups start at a multiple of 4 entries; the group holding `ds` may begin up to 3 entries early and
-        // the one holding `end - 1` may reach up to 3 entries further -- inside the same 16 aligned bytes as a valid
-        // entry, hence mapped; the validity mask drops them
-        const long long A = vec ? (ds & ~3LL) : ds;
-        for (long long c0 = A; c0 < end; c0 += 1024) {
-            const long long e0 = c0 + 4 * lane; // entry of component 0 of this lane's first load; load i is 128 entries on
-            uint4 r[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                r[i] = make_uint4(0, 0, 0, 0);
-                const long long e = e0 + 128 * i;
-                if (e < end) {
-                    if (vec) {
-                        r[i] = __ldg(reinterpret_cast<const uint4 *>(a.db_ids + e));
-                    } else { // arena not 16-byte aligned: one id at a time
-                        r[i].x = __ldg(a.db_ids + e);
-                        if (e + 1 < end) r[i].y = __ldg(a.db_ids + e + 1);
-                        if (e + 2 < end) r[i].z = __ldg(a.db_ids + e + 2);
-                        if (e + 3 < end) r[i].w = __ldg(a.db_ids + e + 3);
-                    }
-                }
-            }
-            const int left = static_cast<int>(min(end - e0, 4096LL));   // entries from e0 to the end of the vector
-            const int skip = static_cast<int>(min(max(ds - e0, 0LL), 4LL)); // > 0 only in the very first load of the vector
-            uint32_t mb = 0;
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                uint32_t nib = bow_maybe(bitmap, bwords, r[i].x) | (bow_maybe(bitmap, bwords, r[i].y) << 1) |
-                               (bow_maybe(bitmap, bwords, r[i].z) << 2) | (bow_maybe(bitmap, bwords, r[i].w) << 3);
-                const int n_valid = min(max(left - 128 * i, 0), 4);
-                nib &= (1u << n_valid) - 1u;
-                if (i == 0) nib &= ~((1u << skip) - 1u);
-                mb |= nib << (4 * i);
-            }
-            if (!__ballot_sync(0xFFFFFFFFu, mb != 0)) continue;
-            // per-load candidate counts of this lane, packed one byte each, and their inclusive prefix over the lanes
-            uint32_t x = mb - ((mb >> 1) & 0x55555555u);
-            x = (x & 0x33333333u) + ((x >> 2) & 0x33333333u); // a popcount per nibble
-            const uint32_t own0 = bow_spread4(x & 0xFFFFu), own1 = bow_spread4(x >> 16);
-            uint32_t in0 = own0, in1 = own1;
-#pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                const uint32_t t0 = __shfl_up_sync(0xFFFFFFFFu, in0, off), t1 = __shfl_up_sync(0xFFFFFFFFu, in1, off);
-                if (lane >= off) {
-                    in0 += t0; // a byte never exceeds 128 (32 lanes x 4)
-                    in1 += t1;
-                }
-            }
-            const uint32_t tot0 = __shfl_sync(0xFFFFFFFFu, in0, 31), tot1 = __shfl_sync(0xFFFFFFFFu, in1, 31);
-            const int sum0 = static_cast<int>(__vsadu4(tot0, 0u)), total = sum0 + static_cast<int>(__vsadu4(tot1, 0u));
-            if (total > 32) {
-                if (n_pend) score = bow_flush(a, qv, table, pend, n_pend, score);
-                n_pend = 0;
-                score = bow_dense_chunk(a, qv, table, bitmap, c0, ds, end, score);
-                continue;
-            }
-            if (n_pend + total > 32) {
-                score = bow_flush(a, qv, table, pend, n_pend, score);
-                n_pend = 0;
-            }
-            // rank of the first candidate of load i of this lane = candidates of the loads before i (all lanes) +
-            // candidates of load i in the lanes below; every byte stays <= 32 here
-            const uint32_t rk0 = tot0 * 0x01010100u + (in0 - own0);
-            const uint32_t rk1 = tot1 * 0x01010100u + static_cast<uint32_t>(sum0) * 0x01010101u + (in1 - own1);
-            uint32_t m = mb;
-            while (m) {
-                const int k = __ffs(m) - 1, i = k >> 2;
-                const uint32_t rk = ((i < 4 ? rk0 : rk1) >> (8 * (i & 3))) & 0xFFu;
-                const uint32_t before = __popc((mb >> (4 * i)) & ((1u << (k & 3)) - 1u));
-                pend[n_pend + rk + before] = e0 + 128 * i + (k & 3);
-                m &= m - 1;
-            }
-            n_pend += total;
-        }
-        if (n_pend) score = bow_flush(a, qv, table, pend, n_pend, score);
+        const double score = bow_score_vector(a, s, ds, end);
         if (lane == 0) a.scores[static_cast<size_t>(q) * a.n_db + j] = __ddiv_rn(-score, 2.0);
     }
+}
+
+// ---- loop-closure keyframe database: the score row of a new keyframe ----
+struct LoopScoreArgs {
+    BowScoreArgs s[2]; // per vocabulary (blockIdx.y): query = the new slot, database = every slot, scores = its row
+    const uint8_t *live;
+};
+
+// grid = (CTAs over the slots, vocabularies).  The new keyframe's slot (written by bow_transform_slots_kernel) against
+// every live slot, itself included, through the same per-vector loop as bow_score_kernel: same bitmap, hash table and
+// summation order, so every score equals plm_bow_score's bit for bit.  Culled slots are skipped and left unwritten.
+__global__ void __launch_bounds__(512) bow_score_row_kernel(LoopScoreArgs r) {
+    const BowScoreArgs &a = r.s[blockIdx.y];
+    const BowScoreSmem s = bow_score_stage(a, 0);
+    const int lane = threadIdx.x & 31;
+    const int warps = blockDim.x >> 5;
+    for (int j = blockIdx.x * warps + (threadIdx.x >> 5); j < a.n_db; j += gridDim.x * warps) {
+        if (!__ldg(r.live + j)) continue;
+        const long long ds = __ldg(a.db_start + j);
+        const double score = bow_score_vector(a, s, ds, ds + max(__ldg(a.db_len + j), 0));
+        if (lane == 0) a.scores[j] = __ddiv_rn(-score, 2.0);
+    }
+}
+
+// insertKFBowVectorPL's blend of the two rows (mapHandler.cpp:3212-3226), every operation rounded on its own (no FMA):
+//   s = 0.0 + (sp * n_pt + sl * n_ls) / n_pl;  s = s + (sp * std_pt + sl * std_ls) / std_pl
+// with n_pl = n_pt + n_ls and std_pl = std_ls + std_pt.  The leading 0.0 + turns a -0.0 score into +0.0.
+__global__ void bow_blend_kernel(const double *__restrict__ sp, const double *__restrict__ sl, int n, double n_pt, double std_pt,
+                                 double n_ls, double std_ls, double *__restrict__ out) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const double n_pl = __dadd_rn(n_pt, n_ls), std_pl = __dadd_rn(std_ls, std_pt);
+    const double p = sp[j], l = sl[j];
+    double s = __dadd_rn(0.0, __ddiv_rn(__dadd_rn(__dmul_rn(p, n_pt), __dmul_rn(l, n_ls)), n_pl));
+    s = __dadd_rn(s, __ddiv_rn(__dadd_rn(__dmul_rn(p, std_pt), __dmul_rn(l, std_ls)), std_pl));
+    out[j] = s;
 }
 
 } // namespace plm

@@ -3305,3 +3305,4 @@ PLM_API int plm_map_gate(plm_ctx *ctx, int is_lines, const double *pf, const int
 
 #include "plm_frames_api.inl"
 #include "plm_shard_api.inl"
+#include "plm_loopdb_api.inl"
