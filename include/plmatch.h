@@ -650,7 +650,10 @@ int64_t plm_loopdb_d2h_bytes(const plm_loopdb *db);
  *   "knn_variant"  -1 = automatic (default: 3 for train sets >= 65 536 rows, 5 for short train sides with >= 2^26 pairs,
  *                  else 1), 0 = plain 8-POPC Hamming, 1 = carry-save 5-POPC, 2 = carry-save 4-POPC with blocked top-2
  *                  update, 3 = 13-LOP3 / 4-POPC in the transformed domain (blocked update), 4 = 3 with three lower-bound
- *                  rows per block, 5 = 13-LOP3 with the per-pair update.
+ *                  rows per block, 5 = 13-LOP3 with the per-pair update, 7 = the tensor-core kernel (int8 tcgen05 MMA,
+ *                  exact) for every single-direction brute force (plm_dev_knn2, plm_knn2, plm_match_nnr, plm_db_knn2);
+ *                  automatic mode takes it for train sets >= 65 536 rows with >= 256 queries.  Environment:
+ *                  PLM_KNN_VARIANT=popc8|csa5|csa4|t13|mix|t13s|umma.
  *   "knn_qpt"      2 = long scans with >= 4096 queries keep two queries per thread (default 1).
  *   "knn_fill"     0 = do not fill the last resident CTA slots / share the second-best bound (default 1).
  *   "frame_fused"  1 = frame sessions and stand-alone frame-sized calls run as ONE launch (frame_fused_kernel, default),
@@ -672,6 +675,9 @@ int plm_set_option(const char *key, int value);
 /* Issue-rate micro-benchmark of the integer pipe on the context's device: giga-instructions/s of
  * independent POPC.32 (*popc_gops) and LOP3.32 (*lop3_gops) per GPU. */
 int plm_measure_int_peaks(plm_ctx *ctx, double *popc_gops, double *lop3_gops);
+/* Rate of back-to-back int8 tensor-core MMAs (tcgen05.mma kind::i8, 128 x 256 x 32, s32 accumulate) on every SM of the
+ * context's device: tera-operations/s (2 per multiply-accumulate) per GPU. */
+int plm_measure_mma_i8_peak(plm_ctx *ctx, double *tops);
 
 #ifdef __cplusplus
 }

@@ -206,6 +206,7 @@ SIGNATURES = {
     "plm_dev_med_desc": (C.c_int, [vp, vp, C.c_int64, vp, vp, C.c_int, vp, vp, vp, vp]),
     "plm_set_option": (C.c_int, [C.c_char_p, C.c_int]),
     "plm_measure_int_peaks": (C.c_int, [vp, f64p, f64p]),
+    "plm_measure_mma_i8_peak": (C.c_int, [vp, f64p]),
 }
 
 _lib = None

@@ -24,6 +24,7 @@
 #include "plm_frame_fused.cuh"
 #include "plm_grid.cuh"
 #include "plm_knn2.cuh"
+#include "plm_knn2_umma.cuh"
 #include "plm_map.cuh"
 #include "plm_reproj.cuh"
 #include "plm_micro.cuh"
@@ -81,6 +82,9 @@ struct plm_ctx {
     bool fused_attr_set = false;
     bool cluster_attr_set = false;
     int knn_occ[2][7] = {{0, 0, 0, 0, 0, 0, 0}, {0, 0, 0, 0, 0, 0, 0}};
+    bool umma_attr_set = false;
+    // set by knn2_umma_kernel / mma_i8_rate_kernel when an MMA completion wait timed out (mapped pinned word)
+    int32_t *umma_err_host = nullptr, *umma_err_dev = nullptr;
     size_t chunked_attr[2] = {0, 0};
     bool rows_attr_set = false;
     bool frame_fused_attr_set = false;
@@ -234,8 +238,12 @@ int g_frame_fused = 1;  // frame sessions run as ONE launch (frame_fused_kernel)
 int g_grid_head = 1;    // map-sized matchGrid: short CTAs at the start of the map (0: uniform rows per CTA, measurement / tests)
 int g_grid_rows = 1;    // map-sized matchGrid uses the row-parallel kernels (0: warp-per-chunk kernels, measurement / tests)
 
-// -1 = automatic (variant 3 for long slices, 1 otherwise); 0..3 force a variant (measurement only)
+// -1 = automatic (the tensor-core kernel for long scans with many queries, variant 3 for other long slices, 1 otherwise);
+// 0..5 force an integer variant, 7 the tensor-core kernel wherever a launch could take it (measurement and tests)
 int g_knn_variant = -2;
+// fewest queries for which a long scan (>= 65 536 train rows) runs on the tensor cores: a group of 256 queries costs the
+// tensor kernel the same whether it is full or not, and at 256 queries it is already 2.6 x faster (DESIGN K1b)
+constexpr int KNN_UMMA_MIN_QUERIES = 256;
 int knn_variant_for(int slice_rows) {
     if (g_knn_variant == -2) {
         const char *e = std::getenv("PLM_KNN_VARIANT");
@@ -246,13 +254,22 @@ int knn_variant_for(int slice_rows) {
         if (e && std::strcmp(e, "t13") == 0) g_knn_variant = 3;
         if (e && std::strcmp(e, "mix") == 0) g_knn_variant = 4;
         if (e && std::strcmp(e, "t13s") == 0) g_knn_variant = 5;
+        if (e && std::strcmp(e, "umma") == 0) g_knn_variant = 7;
         const char *f = std::getenv("PLM_KNN_FILL"); // measurement knob, same as option "knn_fill"
         if (f) g_knn_fill = std::atoi(f) ? 1 : 0;
         const char *q2 = std::getenv("PLM_KNN_QPT");
         if (q2) g_knn_qpt = std::atoi(q2) == 2 ? 2 : 1;
     }
-    if (g_knn_variant >= 0) return g_knn_variant;
+    if (g_knn_variant >= 0 && g_knn_variant != 7) return g_knn_variant;
     return slice_rows >= 2048 ? 3 : 1;
+}
+
+// Single-direction launches (allow_two) of a long scan take the tensor-core kernel (variant 7).
+bool knn_use_umma(int n1, long long n2, bool allow_two) {
+    (void)knn_variant_for(0); // reads PLM_KNN_VARIANT on first use
+    if (!allow_two || n2 <= 0) return false;
+    if (g_knn_variant == 7) return true;
+    return g_knn_variant < 0 && n2 >= 65536 && n1 >= KNN_UMMA_MIN_QUERIES;
 }
 
 // CTAs of the brute-force kernel that are resident on one SM (per CTA width and variant).
@@ -289,10 +306,25 @@ int knn_ctas_per_sm(plm_ctx *ctx, int threads, int variant) {
 // still spreads over the whole chip.
 KnnPlan plan_knn(plm_ctx *ctx, int n1, long long n2, bool allow_two = false) {
     KnnPlan p;
+    if (knn_use_umma(n1, n2, allow_two)) {
+        // one CTA per SM, each owning an equal contiguous share of the (query group, 128-row unit) list; n_workers =
+        // the most CTAs any query group is spread over (knn2_umma_kernel writes the slots a group does not use)
+        p.threads = p.qpb = plm::KNN_UMMA_THREADS;
+        p.unit_rows = plm::KNN_UMMA_ROWS;
+        const long long groups = std::max(1, (n1 + p.qpb - 1) / p.qpb), units = (n2 + p.unit_rows - 1) / p.unit_rows;
+        const long long total = groups * units, ctas = std::min<long long>(ctx->sm_count, total);
+        p.n_units = static_cast<int>(units);
+        p.n_workers = 1;
+        for (long long g = 0; g < groups; ++g)
+            p.n_workers = static_cast<int>(std::max<long long>(p.n_workers, plm::umma_cta_of(g * units + units - 1, total, ctas) -
+                                                                                  plm::umma_cta_of(g * units, total, ctas) + 1));
+        p.share_thr = true;
+        return p;
+    }
     p.threads = (n1 >= 4096) ? 128 : 64;
     int variant = knn_variant_for(n2 >= 65536 ? 4096 : 64);
     // a short train side with a lot of work is launched with variant 5 (launch_knn_slices): plan the workers for it
-    if (variant == 1 && g_knn_variant < 0 && n2 >= 64 && static_cast<long long>(n1) * n2 >= (1ll << 26)) variant = 5;
+    if (variant == 1 && (g_knn_variant < 0 || g_knn_variant == 7) && n2 >= 64 && static_cast<long long>(n1) * n2 >= (1ll << 26)) variant = 5;
     // long scans with many queries: two queries per thread (variant 6), single-direction launches only
     if (allow_two && variant == 3 && g_knn_qpt == 2 && p.threads == 128) variant = 6;
     p.qpb = (variant == 6) ? 2 * p.threads : p.threads;
@@ -313,6 +345,29 @@ KnnPlan plan_knn(plm_ctx *ctx, int n1, long long n2, bool allow_two = false) {
     return p;
 }
 
+// The mapped pinned word the tensor-core kernels raise when an MMA completion wait runs past the spin limit (option
+// "peer_spin_ms").  Such a launch's results are undefined, so from then on every tensor-core launch of the context fails
+// instead of returning them.
+int umma_error_word(plm_ctx *ctx) {
+    if (!ctx->umma_err_host) {
+        int32_t *h = nullptr;
+        void *d = nullptr;
+        CU_TRY(cudaHostAlloc(reinterpret_cast<void **>(&h), sizeof(int32_t), cudaHostAllocMapped));
+        *h = 0;
+        const cudaError_t e = cudaHostGetDevicePointer(&d, h, 0);
+        if (e != cudaSuccess) {
+            cudaFreeHost(h);
+            return fail(PLM_E_CUDA, std::string("cudaHostGetDevicePointer: ") + cudaGetErrorString(e));
+        }
+        ctx->umma_err_host = h;
+        ctx->umma_err_dev = static_cast<int32_t *>(d);
+    }
+    if (*reinterpret_cast<volatile int32_t *>(ctx->umma_err_host) != 0)
+        return fail(PLM_E_CUDA, "tensor-core brute force: an MMA completion wait timed out in an earlier launch on this context "
+                                "(its results are undefined); destroy the context");
+    return PLM_OK;
+}
+
 int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threads) {
     long long total = 0;
     for (int i = 0; i < n_tasks; ++i) {
@@ -322,13 +377,20 @@ int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threa
         total += c;
     }
     if (n_tasks == 1) tp.cta_split = static_cast<int>(total);
+    // planned for the tensor-core kernel (plan_knn: single task, 256 queries per CTA)
+    const bool umma = n_tasks == 1 && threads == plm::KNN_UMMA_THREADS;
+    if (umma) {
+        const long long units = tp.t[0].n_units, groups = (tp.t[0].n1 + threads - 1) / threads;
+        total = std::min<long long>(ctx->sm_count, groups * units);
+        tp.cta_split = static_cast<int>(total);
+    }
     if (total == 0) return PLM_OK;
     if (total > INT_MAX) return fail(PLM_E_UNSUPPORTED, "too many query blocks");
     const dim3 grid(static_cast<unsigned>(total), 1, 1);
     int min_rows = INT_MAX;
     for (int i = 0; i < n_tasks; ++i) min_rows = std::min<long long>(min_rows, std::min<long long>(tp.t[i].n2, INT_MAX));
     int variant = knn_variant_for(min_rows >= 65536 ? 4096 : 64);
-    if (variant == 1 && g_knn_variant < 0 && min_rows >= 64) {
+    if (variant == 1 && (g_knn_variant < 0 || g_knn_variant == 7) && min_rows >= 64) {
         // a short train side but a lot of work (the match fallback of the local map, 200 000 x 600 in both directions):
         // the 13-LOP3 distance with the per-pair update (variant 5) -- a few per cent there (0.369 -> 0.356 ms, plan_knn sizes the workers for it); frame-sized calls keep
         // variant 1, whose stages need no in-place transform
@@ -337,7 +399,15 @@ int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threa
         if (pairs >= (1ll << 26)) variant = 5;
     }
     if (n_tasks == 1 && tp.t[0].threads == 2 * threads) variant = 6; // planned with two queries per thread
-    if (variant >= 2 && g_knn_fill) {
+    if (umma) {
+        if (!ctx->umma_attr_set) {
+            CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_SMEM));
+            ctx->umma_attr_set = true;
+        }
+        const int st = umma_error_word(ctx);
+        if (st != PLM_OK) return st;
+    }
+    if (umma || (variant >= 2 && g_knn_fill)) {
         // the shared second-best bounds live behind each task's partial results (build_knn_task reserved the room)
         for (int i = 0; i < n_tasks; ++i) {
             plm::KnnTask &t = tp.t[i];
@@ -358,7 +428,9 @@ int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threa
         CU_TRY(cudaEventRecord(ev.first, ctx->stream));
     }
 #define PLM_KNN_LAUNCH(T, V) plm::knn2_slice_kernel<T, V><<<grid, T, 0, ctx->stream>>>(tp)
-    if (threads == 128) {
+    if (umma) {
+        plm::knn2_umma_kernel<<<grid, plm::KNN_UMMA_THREADS, plm::KNN_UMMA_SMEM, ctx->stream>>>(tp.t[0], ctx->umma_err_dev, g_peer_spin_ticks);
+    } else if (threads == 128) {
         if (variant == 6) PLM_KNN_LAUNCH(128, 6);
         else if (variant == 5) PLM_KNN_LAUNCH(128, 5);
         else if (variant == 4) PLM_KNN_LAUNCH(128, 4);
@@ -420,7 +492,7 @@ int check_desc(const uint8_t *d, int n, size_t step) {
 PLM_API int plm_set_option(const char *key, int value) {
     if (!key) return fail(PLM_E_INVALID, "null key");
     if (std::strcmp(key, "knn_variant") == 0) {
-        g_knn_variant = (value >= 0 && value <= 5) ? value : -1;
+        g_knn_variant = ((value >= 0 && value <= 5) || value == 7) ? value : -1;
         return PLM_OK;
     }
     if (std::strcmp(key, "peer_spin_ms") == 0) {
@@ -539,6 +611,7 @@ PLM_API int plm_ctx_destroy(plm_ctx *ctx) {
     if (ctx->d_buf) cudaFree(ctx->d_buf);
     if (ctx->d_aux) cudaFree(ctx->d_aux);
     if (ctx->h_buf) cudaFreeHost(ctx->h_buf);
+    if (ctx->umma_err_host) cudaFreeHost(ctx->umma_err_host);
     if (g_tls.ctx == ctx) g_tls.ctx = nullptr;
     delete ctx;
     return PLM_OK;
@@ -2479,6 +2552,35 @@ PLM_API int plm_measure_int_peaks(plm_ctx *ctx, double *popc_gops, double *lop3_
     cudaEventDestroy(e1);
     if (popc_gops) *popc_gops = out[0];
     if (lop3_gops) *lop3_gops = out[1];
+    return PLM_OK;
+}
+
+PLM_API int plm_measure_mma_i8_peak(plm_ctx *ctx, double *tops) {
+    int st = resolve_ctx(ctx);
+    if (st != PLM_OK) return st;
+    if ((st = umma_error_word(ctx)) != PLM_OK) return st;
+    CU_TRY(cudaFuncSetAttribute(plm::mma_i8_rate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_RATE_SMEM));
+    cudaEvent_t e0, e1;
+    CU_TRY(cudaEventCreate(&e0));
+    CU_TRY(cudaEventCreate(&e1));
+    const int iters = 16384; // 8 MMAs of 128 x 256 x 32 each: ~10 ms at the data-sheet rate
+    float best_ms = 1e30f;
+    for (int rep = 0; rep < 4; ++rep) {
+        CU_TRY(cudaEventRecord(e0, ctx->stream));
+        plm::mma_i8_rate_kernel<<<ctx->sm_count, 128, plm::KNN_UMMA_RATE_SMEM, ctx->stream>>>(iters, ctx->umma_err_dev, g_peer_spin_ticks);
+        ctx->launches++;
+        CU_TRY(cudaGetLastError());
+        CU_TRY(cudaEventRecord(e1, ctx->stream));
+        CU_TRY(cudaEventSynchronize(e1));
+        float ms = 0.f;
+        CU_TRY(cudaEventElapsedTime(&ms, e0, e1));
+        if (rep > 0) best_ms = std::min(best_ms, ms);
+    }
+    cudaEventDestroy(e0);
+    cudaEventDestroy(e1);
+    if ((st = umma_error_word(ctx)) != PLM_OK) return st;
+    const double ops = 2.0 * ctx->sm_count * double(iters) * 8.0 * 128.0 * 256.0 * 32.0;
+    if (tops) *tops = ops / (best_ms * 1e-3) * 1e-12;
     return PLM_OK;
 }
 

@@ -79,6 +79,12 @@ class Context:
         L.check(self._lib.plm_measure_int_peaks(self._h, C.byref(p), C.byref(l)), "plm_measure_int_peaks")
         return p.value, l.value
 
+    def measure_mma_i8_peak(self) -> float:
+        """Int8 tensor-core MMA rate of this device, tera-operations/s (plm_measure_mma_i8_peak)."""
+        t = C.c_double(0)
+        L.check(self._lib.plm_measure_mma_i8_peak(self._h, C.byref(t)), "plm_measure_mma_i8_peak")
+        return t.value
+
     def close(self):
         if self._h:
             self._lib.plm_ctx_destroy(self._h)
