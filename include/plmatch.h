@@ -678,6 +678,10 @@ int plm_measure_int_peaks(plm_ctx *ctx, double *popc_gops, double *lop3_gops);
 /* Rate of back-to-back int8 tensor-core MMAs (tcgen05.mma kind::i8, 128 x 256 x 32, s32 accumulate) on every SM of the
  * context's device: tera-operations/s (2 per multiply-accumulate) per GPU. */
 int plm_measure_mma_i8_peak(plm_ctx *ctx, double *tops);
+/* Rate of back-to-back int8 tensor-core MMAs of shape 128 x n x 32 (n = 128 or 256) on every SM, tera-operations/s per
+ * GPU.  with_stores != 0: three more warps per SM keep storing to shared memory meanwhile, as the expansion of the
+ * tensor-core brute force does.  plm_measure_mma_i8_peak is n = 256 without stores. */
+int plm_measure_mma_i8_rate(plm_ctx *ctx, int n, int with_stores, double *tops);
 
 #ifdef __cplusplus
 }

@@ -207,6 +207,7 @@ SIGNATURES = {
     "plm_set_option": (C.c_int, [C.c_char_p, C.c_int]),
     "plm_measure_int_peaks": (C.c_int, [vp, f64p, f64p]),
     "plm_measure_mma_i8_peak": (C.c_int, [vp, f64p]),
+    "plm_measure_mma_i8_rate": (C.c_int, [vp, C.c_int, C.c_int, f64p]),
 }
 
 _lib = None

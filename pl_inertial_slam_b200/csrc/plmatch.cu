@@ -242,7 +242,7 @@ int g_grid_rows = 1;    // map-sized matchGrid uses the row-parallel kernels (0:
 // 0..5 force an integer variant, 7 the tensor-core kernel wherever a launch could take it (measurement and tests)
 int g_knn_variant = -2;
 // fewest queries for which a long scan (>= 65 536 train rows) runs on the tensor cores: a group of 256 queries costs the
-// tensor kernel the same whether it is full or not, and at 256 queries it is already 2.6 x faster (DESIGN K1b)
+// tensor kernel the same whether it is full or not, and at 256 queries it is already 3.1 x faster (DESIGN K1b)
 constexpr int KNN_UMMA_MIN_QUERIES = 256;
 int knn_variant_for(int slice_rows) {
     if (g_knn_variant == -2) {
@@ -429,7 +429,7 @@ int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threa
     }
 #define PLM_KNN_LAUNCH(T, V) plm::knn2_slice_kernel<T, V><<<grid, T, 0, ctx->stream>>>(tp)
     if (umma) {
-        plm::knn2_umma_kernel<<<grid, plm::KNN_UMMA_THREADS, plm::KNN_UMMA_SMEM, ctx->stream>>>(tp.t[0], ctx->umma_err_dev, g_peer_spin_ticks);
+        plm::knn2_umma_kernel<<<grid, plm::KNN_UMMA_CTA_THREADS, plm::KNN_UMMA_SMEM, ctx->stream>>>(tp.t[0], ctx->umma_err_dev, g_peer_spin_ticks);
     } else if (threads == 128) {
         if (variant == 6) PLM_KNN_LAUNCH(128, 6);
         else if (variant == 5) PLM_KNN_LAUNCH(128, 5);
@@ -2555,19 +2555,22 @@ PLM_API int plm_measure_int_peaks(plm_ctx *ctx, double *popc_gops, double *lop3_
     return PLM_OK;
 }
 
-PLM_API int plm_measure_mma_i8_peak(plm_ctx *ctx, double *tops) {
+PLM_API int plm_measure_mma_i8_rate(plm_ctx *ctx, int n, int with_stores, double *tops) {
+    if (n != 128 && n != 256) return fail(PLM_E_INVALID, "plm_measure_mma_i8_rate: n must be 128 or 256");
     int st = resolve_ctx(ctx);
     if (st != PLM_OK) return st;
     if ((st = umma_error_word(ctx)) != PLM_OK) return st;
-    CU_TRY(cudaFuncSetAttribute(plm::mma_i8_rate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_RATE_SMEM));
+    void (*kern)(int, int32_t *, long long) = n == 256 ? (with_stores ? plm::mma_i8_rate_kernel<256, true> : plm::mma_i8_rate_kernel<256, false>)
+                                                       : (with_stores ? plm::mma_i8_rate_kernel<128, true> : plm::mma_i8_rate_kernel<128, false>);
+    CU_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_RATE_SMEM));
     cudaEvent_t e0, e1;
     CU_TRY(cudaEventCreate(&e0));
     CU_TRY(cudaEventCreate(&e1));
-    const int iters = 16384; // 8 MMAs of 128 x 256 x 32 each: ~10 ms at the data-sheet rate
+    const int iters = 16384 * (256 / n); // 8 MMAs of 128 x n x 32 each: ~10 ms at the data-sheet rate
     float best_ms = 1e30f;
     for (int rep = 0; rep < 4; ++rep) {
         CU_TRY(cudaEventRecord(e0, ctx->stream));
-        plm::mma_i8_rate_kernel<<<ctx->sm_count, 128, plm::KNN_UMMA_RATE_SMEM, ctx->stream>>>(iters, ctx->umma_err_dev, g_peer_spin_ticks);
+        kern<<<ctx->sm_count, 128, plm::KNN_UMMA_RATE_SMEM, ctx->stream>>>(iters, ctx->umma_err_dev, g_peer_spin_ticks);
         ctx->launches++;
         CU_TRY(cudaGetLastError());
         CU_TRY(cudaEventRecord(e1, ctx->stream));
@@ -2579,10 +2582,20 @@ PLM_API int plm_measure_mma_i8_peak(plm_ctx *ctx, double *tops) {
     cudaEventDestroy(e0);
     cudaEventDestroy(e1);
     if ((st = umma_error_word(ctx)) != PLM_OK) return st;
-    const double ops = 2.0 * ctx->sm_count * double(iters) * 8.0 * 128.0 * 256.0 * 32.0;
+    const double ops = 2.0 * ctx->sm_count * double(iters) * 8.0 * 128.0 * double(n) * 32.0;
     if (tops) *tops = ops / (best_ms * 1e-3) * 1e-12;
     return PLM_OK;
 }
+
+PLM_API int plm_measure_mma_i8_peak(plm_ctx *ctx, double *tops) { return plm_measure_mma_i8_rate(ctx, 256, 0, tops); }
+
+#ifdef PLM_UMMA_STAMPS
+// debug builds: the role stamps of the last knn2_umma_kernel launch, [KNN_UMMA_STAMP_CTAS][4 roles][3] (see the kernel)
+extern "C" __attribute__((visibility("default"))) int plm_debug_umma_stamps(long long *out) {
+    cudaDeviceSynchronize();
+    return cudaMemcpyFromSymbol(out, plm::g_umma_stamps, sizeof(plm::g_umma_stamps)) == cudaSuccess ? 0 : -1;
+}
+#endif
 
 // ---------------------------------------------------------------------------------------------
 // Batched replay

@@ -85,6 +85,13 @@ class Context:
         L.check(self._lib.plm_measure_mma_i8_peak(self._h, C.byref(t)), "plm_measure_mma_i8_peak")
         return t.value
 
+    def measure_mma_i8_rate(self, n: int = 256, with_stores: bool = False) -> float:
+        """Int8 MMA rate at 128 x n x 32 (n = 128 or 256), optionally with concurrent shared-memory stores, TOPS
+        (plm_measure_mma_i8_rate)."""
+        t = C.c_double(0)
+        L.check(self._lib.plm_measure_mma_i8_rate(self._h, n, 1 if with_stores else 0, C.byref(t)), "plm_measure_mma_i8_rate")
+        return t.value
+
     def close(self):
         if self._h:
             self._lib.plm_ctx_destroy(self._h)

@@ -6,8 +6,12 @@ tensor-core kernel (variant 7, int8 tcgen05 MMA), alternating in one process.
 * config 5 on one GPU: 6400 queries x 16 M rows through plm_dev_knn2 (slice kernel + merge), a 256 MiB L2 flush
   between calls, CUDA events around each call; `--rounds` rounds of `--calls` calls per kernel, alternating;
 * the keys of both kernels compared on every call of the last round;
-* the int8 MMA rate of the card measured in the same run (plm_measure_mma_i8_peak) and the integer-pipe peaks
-  (plm_measure_int_peaks), so that the tensor kernel's MAC/s can be set against a measured peak;
+* the int8 MMA rate of the card measured in the same run (plm_measure_mma_i8_rate): 128 x 256 x 32 (the peak) and
+  128 x 128 x 32 (the shape the tensor kernel issues), each alone and with concurrent shared-memory stores as the
+  expansion makes them; and the integer-pipe peaks (plm_measure_int_peaks), so that the tensor kernel's MAC/s can be
+  set against a measured rate;
+* with a library built with PLM_BUILD_DEFINES=-DPLM_UMMA_STAMPS: the per-role cycle stamps of the tensor kernel at the
+  bench shape (SM cycles per unit, and the share of it each role spent waiting), which show the role that bounds it;
 * the query count at which the tensor kernel overtakes the integer one (2 M rows, n1 = 256 ... 4096).
 
     python tools/bench_knn_tensor.py --out profiles/r4_knn_tensor_b200.json
@@ -34,6 +38,23 @@ def card_info() -> dict:
         return dict(zip(q.split(","), [x.strip() for x in out.split(",")]))
     except (OSError, subprocess.SubprocessError) as e:
         return {"error": repr(e)}
+
+
+def role_stamps(lib, call) -> dict:
+    """Per-role SM cycles of knn2_umma_kernel from a PLM_UMMA_STAMPS build: one call at the bench shape, then per role
+    the median over CTAs of cycles per unit and of the share of its time spent in mbarrier waits."""
+    import ctypes as C
+    call()
+    buf = (C.c_longlong * (160 * 4 * 3))()
+    assert lib.plm_debug_umma_stamps(buf) == 0
+    a = np.frombuffer(buf, dtype=np.int64).reshape(160, 4, 3)
+    a = a[a[:, 0, 2] > 0]
+    out = {}
+    for r, name in enumerate(("readout", "expander", "producer", "mma")):
+        total, waited, units = a[:, r, 0].astype(float), a[:, r, 1].astype(float), a[:, r, 2].astype(float)
+        out[name] = {"cycles_per_unit_median": float(np.median(total / units)),
+                     "wait_share_median": float(np.median(waited / total)), "units_median": float(np.median(units))}
+    return out
 
 
 def main():
@@ -77,6 +98,8 @@ def main():
 
     card_before = card_info()
     mma_tops = ops.ctx.measure_mma_i8_peak()
+    mma_rates = {f"n{n}{'_with_stores' if sts else ''}": ops.ctx.measure_mma_i8_rate(n, sts)
+                 for n in (256, 128) for sts in (False, True)}
     popc_gops, lop3_gops = ops.ctx.measure_int_peaks()
     times = {k: [] for k in arms}
     equal = None
@@ -110,12 +133,16 @@ def main():
             ms, _ = run(v, q[:n1], rows2, 3)
             row[name + "_ms"] = float(np.median(ms))
         sweep.append(row)
+    stamps = role_stamps(lib, lambda: run(7, q, db, 1)) if hasattr(lib, "plm_debug_umma_stamps") else None
     lib.plm_set_option(b"knn_variant", -1)
 
     out = {"card_before": card_before, "card_after": card_after,
            "shape": {"queries": n_q, "db_rows": n_rows, "K_bits": 256, "pairs_per_call": pairs, "macs_per_call": macs},
            "call": "plm_dev_knn2 (slice kernel + merge kernel), L2 flushed (256 MiB write) before each call",
            "measured_peaks": {"int8_mma_tops": mma_tops, "popc_gops": popc_gops, "lop3_gops": lop3_gops},
+           "int8_mma_tops_by_shape": mma_rates,
+           "tensor_share_of_n128_rate": res["tensor_umma"]["int8_tops_achieved"] / mma_rates["n128"],
+           "tensor_role_stamps": stamps,
            "keys_equal_last_round": equal, "arms": res, "n1_crossover_2m_rows": sweep}
     text = json.dumps(out, indent=1)
     print(text)
