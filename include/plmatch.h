@@ -229,7 +229,10 @@ int plm_batch_set_match(plm_batch *b, const uint8_t *arena, int64_t n_rows, cons
  * valid and its rows may be rewritten between runs): the per-keyframe-pair form of loop-closure matching -- StVO::match
  * of one query keyframe against every keyframe of a resident database (isLoopClosure, mapHandler.cpp:3325-3378, at
  * scale; SURVEY 8d "Mode A").  Prepare once with the query rows in a fixed slot of the arena, then per query: rewrite
- * the slot, plm_batch_run, plm_batch_fetch.  m12_arena may be NULL: every match vector then starts at -1. */
+ * the slot, plm_batch_run, plm_batch_fetch.  m12_arena may be NULL: every match vector then starts at -1.
+ * When every live job shares one query range (off1, n1) -- this form -- option "batch_umma" = 1 makes both directions
+ * of every pair come from one int8 tensor-core product per 256 query rows x 128 train rows (knn2_umma_pairs_kernel);
+ * results are identical either way, and so is the number of launches per run. */
 int plm_batch_set_match_dev(plm_batch *b, const void *arena_dev, int64_t n_rows, const plm_pair_job *jobs,
                             int n_jobs, float nnr, int best_lr, const int32_t *m12_arena, int64_t n_m);
 
@@ -636,7 +639,9 @@ int plm_loopdb_bow(plm_loopdb *db, int kf_idx, int which, uint32_t *ids, double 
  * points of kf0 against points of kf1[k] with nnr_p -> count_pt[k], m12_pt[k * n_p(kf0) ..]; lines with nnr_l ->
  * count_ls[k], m12_ls[k * n_l(kf0) ..] (either match array may be NULL).  Results equal plm_match's on the same rows,
  * including a side with 0 or 1 rows: count 0 and every entry -1 (the reference skips an empty side).  Every keyframe
- * must be live (PLM_E_INVALID otherwise, before any work). */
+ * must be live (PLM_E_INVALID otherwise, before any work).  Points and lines run as one batch when nnr_p == nnr_l;
+ * with option "batch_umma" = 1 (the tensor-core path of plm_batch_set_match_dev) each kind gets a batch of its own,
+ * whose jobs share kf0's rows as the query range. */
 int plm_loopdb_match(plm_loopdb *db, int kf0, const int32_t *kf1, int n_pairs, float nnr_p, float nnr_l, int best_lr,
                      int32_t *count_pt, int32_t *count_ls, int32_t *m12_pt, int32_t *m12_ls);
 /* Keyframes inserted (culled ones included). */
@@ -654,6 +659,11 @@ int64_t plm_loopdb_d2h_bytes(const plm_loopdb *db);
  *                  exact) for every single-direction brute force (plm_dev_knn2, plm_knn2, plm_match_nnr, plm_db_knn2);
  *                  automatic mode takes it for train sets >= 65 536 rows with >= 256 queries.  Environment:
  *                  PLM_KNN_VARIANT=popc8|csa5|csa4|t13|mix|t13s|umma.
+ *   "batch_umma"   batches of plm_batch_set_match / _dev (and plm_loopdb_match) whose live jobs share one query range:
+ *                  1 = both directions of every pair from one int8 tensor-core product (knn2_umma_pairs_kernel),
+ *                  0 = the integer list kernels, -1 = automatic (default; today the integer list kernels, which measured
+ *                  faster at the loop-closure shapes, DESIGN K1c).  Read when the batch is prepared.  Forcing
+ *                  "knn_variant" 0-5 keeps the integer kernels.
  *   "knn_qpt"      2 = long scans with >= 4096 queries keep two queries per thread (default 1).
  *   "knn_fill"     0 = do not fill the last resident CTA slots / share the second-best bound (default 1).
  *   "frame_fused"  1 = frame sessions and stand-alone frame-sized calls run as ONE launch (frame_fused_kernel, default),

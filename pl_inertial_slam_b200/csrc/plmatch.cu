@@ -25,6 +25,7 @@
 #include "plm_grid.cuh"
 #include "plm_knn2.cuh"
 #include "plm_knn2_umma.cuh"
+#include "plm_knn2_umma_pairs.cuh"
 #include "plm_map.cuh"
 #include "plm_reproj.cuh"
 #include "plm_micro.cuh"
@@ -83,6 +84,7 @@ struct plm_ctx {
     bool cluster_attr_set = false;
     int knn_occ[2][7] = {{0, 0, 0, 0, 0, 0, 0}, {0, 0, 0, 0, 0, 0, 0}};
     bool umma_attr_set = false;
+    bool umma_pairs_attr_set = false;
     // set by knn2_umma_kernel / mma_i8_rate_kernel when an MMA completion wait timed out (mapped pinned word)
     int32_t *umma_err_host = nullptr, *umma_err_dev = nullptr;
     size_t chunked_attr[2] = {0, 0};
@@ -270,6 +272,18 @@ bool knn_use_umma(int n1, long long n2, bool allow_two) {
     if (!allow_two || n2 <= 0) return false;
     if (g_knn_variant == 7) return true;
     return g_knn_variant < 0 && n2 >= 65536 && n1 >= KNN_UMMA_MIN_QUERIES;
+}
+
+// Batches whose live jobs all share one query range (a loop-closure batch: one query keyframe against many) can run
+// both directions of every pair from one tensor-core product (K1c, knn2_umma_pairs_kernel).  Option "batch_umma": -1
+// automatic (default), 0 never, 1 every such batch.  Automatic selection keeps the integer list kernels: the pairs
+// kernel is bound by its readout (~16.6 k SM cycles per unit, ~14.9 k of them without direction 21) and measured slower
+// at 800 x 2000 x 800, 800 x 20 000 x 800 and 200 x 2000 x 200 (tools/bench_mode_a_tensor.py, DESIGN K1c).
+int g_batch_umma = -1;
+bool batch_use_umma(int n1, long long live_rows) {
+    (void)knn_variant_for(0); // reads PLM_KNN_VARIANT on first use
+    if (n1 <= 0 || live_rows <= 0 || (g_knn_variant >= 0 && g_knn_variant <= 5)) return false; // a forced integer variant
+    return g_batch_umma == 1;
 }
 
 // CTAs of the brute-force kernel that are resident on one SM (per CTA width and variant).
@@ -493,6 +507,10 @@ PLM_API int plm_set_option(const char *key, int value) {
     if (!key) return fail(PLM_E_INVALID, "null key");
     if (std::strcmp(key, "knn_variant") == 0) {
         g_knn_variant = ((value >= 0 && value <= 5) || value == 7) ? value : -1;
+        return PLM_OK;
+    }
+    if (std::strcmp(key, "batch_umma") == 0) {
+        g_batch_umma = (value == 0 || value == 1) ? value : -1;
         return PLM_OK;
     }
     if (std::strcmp(key, "peer_spin_ms") == 0) {
@@ -2612,6 +2630,9 @@ struct plm_batch {
     int n_slice_ctas = 0, n_merge_ctas = 0, n_x_ctas = 0;
     float nnr = 0.f;
     int best_lr = 0;
+    // shared-query batches on the tensor cores (K1c): the kernel's parameters, its grid (0: integer list kernels)
+    plm::PairsTask ptask;
+    int n_umma_ctas = 0;
     // grid
     size_t o_gjobs = 0;
     plm::GridParams gp;
@@ -2702,7 +2723,10 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
     std::vector<int64_t> m21_off(static_cast<size_t>(n_jobs), 0);
     int64_t m21_rows = 0;
     size_t part_bytes = 0;
-    long long total_qblocks = 0;
+    long long total_qblocks = 0, live_rows = 0;
+    int64_t q_off = -1;
+    int q_n = -1;
+    bool shared_query = true; // every live job has the same query range (a loop-closure batch)
     for (int j = 0; j < n_jobs; ++j) {
         const plm_pair_job &jb = jobs[j];
         if (jb.n1 < 0 || jb.n2 < 0 || jb.off1 < 0 || jb.off2 < 0 || jb.off_m < 0 || jb.off1 + jb.n1 > n_rows ||
@@ -2711,10 +2735,57 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
         if (jb.n2 < 2 || (best_lr && jb.n1 < 2)) continue;
         total_qblocks += (jb.n1 + BATCH_THREADS - 1) / BATCH_THREADS;
         if (best_lr) total_qblocks += (jb.n2 + BATCH_THREADS - 1) / BATCH_THREADS;
+        if (q_n < 0) {
+            q_off = jb.off1;
+            q_n = jb.n1;
+        }
+        shared_query = shared_query && jb.off1 == q_off && jb.n1 == q_n;
+        live_rows += jb.n2;
+    }
+    // Shared-query batches on the tensor cores (K1c): one (query group of 256, unit of <= 128 rows of one job) work list
+    // over one CTA per SM.  The per-job tasks below keep their meaning for the merge and the mutual check; only their
+    // partials change shape: the 12 task of job j has one slot per piece (the CTAs a (group, job) run is cut over), the
+    // 21 task one slot per query group.  Partial memory is sum_j (slots_j * n1 + groups * n2_j) * 16 B -- for 20 000
+    // keyframes x 800 rows against an 800-row query (4 groups) ~0.26 + 1.02 GB, against (n1 + n2_j) * 16 B per job,
+    // ~0.51 GB, on the integer list path (one slice per direction at that size).
+    const bool umma = shared_query && q_n > 0 && batch_use_umma(q_n, live_rows);
+    const int groups = umma ? (q_n + plm::KNN_UMMA_THREADS - 1) / plm::KNN_UMMA_THREADS : 0;
+    std::vector<plm::PairsJob> pjobs;
+    std::vector<int2> units;
+    std::vector<int> slots12(static_cast<size_t>(n_jobs), 0);
+    long long umma_ctas = 0;
+    if (umma) {
+        long long n_units = 0;
+        for (int j = 0; j < n_jobs; ++j)
+            if (!(jobs[j].n2 < 2 || (best_lr && jobs[j].n1 < 2))) n_units += (jobs[j].n2 + plm::KNN_UMMA_ROWS - 1) / plm::KNN_UMMA_ROWS;
+        if (n_units > INT_MAX / 2) return fail(PLM_E_UNSUPPORTED, "batch too large for the tensor-core path");
+        const long long total = groups * n_units;
+        umma_ctas = std::min<long long>(ctx->sm_count, total);
+        units.reserve(static_cast<size_t>(n_units));
+        for (int j = 0; j < n_jobs; ++j) {
+            const plm_pair_job &jb = jobs[j];
+            if (jb.n2 < 2 || (best_lr && jb.n1 < 2)) continue;
+            plm::PairsJob p;
+            std::memset(&p, 0, sizeof(p));
+            p.train_off = jb.off2;
+            p.n2 = jb.n2;
+            p.unit0 = static_cast<int>(units.size());
+            p.n_units = (jb.n2 + plm::KNN_UMMA_ROWS - 1) / plm::KNN_UMMA_ROWS;
+            for (int u = 0; u < p.n_units; ++u) units.push_back(make_int2(static_cast<int>(pjobs.size()), u * plm::KNN_UMMA_ROWS));
+            // slots of the 12 task: the most CTAs one (group, job) run is spread over (the kernel writes the unused ones)
+            p.n_slots12 = 1;
+            for (long long g = 0; g < groups; ++g) {
+                const long long first = g * n_units + p.unit0, last = first + p.n_units - 1;
+                p.n_slots12 = static_cast<int>(std::max<long long>(p.n_slots12, plm::umma_cta_of(last, total, umma_ctas) - plm::umma_cta_of(first, total, umma_ctas) + 1));
+            }
+            slots12[j] = p.n_slots12;
+            pjobs.push_back(p);
+        }
     }
     // slices per direction: enough CTAs for a few waves when the batch is small, 1 when it is large
     const long long target = static_cast<long long>(ctx->sm_count) * 16;
     const int want_slices = static_cast<int>(std::max<long long>(1, target / std::max<long long>(1, total_qblocks)));
+    std::vector<int> task12(static_cast<size_t>(n_jobs), -1); // K1c: the job's tasks (12, and 21 right after it)
     for (int j = 0; j < n_jobs; ++j) {
         const plm_pair_job &jb = jobs[j];
         if (jb.n2 < 2 || (best_lr && jb.n1 < 2)) {
@@ -2723,14 +2794,20 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
         }
         m21_off[j] = m21_rows;
         if (best_lr) m21_rows += jb.n2;
+        task12[j] = static_cast<int>(tasks.size());
         for (int dir = 0; dir <= best_lr; ++dir) {
             plm::KnnTask t;
             std::memset(&t, 0, sizeof(t));
             const int nq = dir ? jb.n2 : jb.n1, nt = dir ? jb.n1 : jb.n2;
             int slices = std::min(want_slices, std::max(1, (nt + 63) / 64)); // workers of this task
-            const int rows = std::min(plm::KNN_STAGE_ROWS, ((nt + slices - 1) / slices + 63) / 64 * 64);
-            const int units = std::max(1, (nt + rows - 1) / rows);
+            int rows = std::min(plm::KNN_STAGE_ROWS, ((nt + slices - 1) / slices + 63) / 64 * 64);
+            int units = std::max(1, (nt + rows - 1) / rows);
             slices = std::min(slices, units);
+            if (umma) { // partial slots as knn2_umma_pairs_kernel writes them; unit fields are informative only
+                slices = dir ? groups : slots12[j];
+                rows = plm::KNN_UMMA_ROWS;
+                units = (jb.n2 + rows - 1) / rows;
+            }
             t.n1 = nq;
             t.n2 = nt;
             t.unit_rows = rows;
@@ -2747,7 +2824,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
             part_bytes += align_up(size_t(slices) * nq * sizeof(ulonglong2));
             const int task_id = static_cast<int>(tasks.size());
             for (int qb = 0; qb * BATCH_THREADS < nq; ++qb) {
-                for (int s = 0; s < slices; ++s) cta_map.push_back(make_int4(task_id, qb, s, 0));
+                if (!umma)
+                    for (int s = 0; s < slices; ++s) cta_map.push_back(make_int4(task_id, qb, s, 0));
                 merge_map.push_back(make_int2(task_id, qb * BATCH_THREADS));
             }
             tasks.push_back(t);
@@ -2777,6 +2855,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
     b->o_xmap = L.add(xmap.size() * sizeof(int2));
     b->m21_bytes = size_t(m21_rows) * 4;
     b->o_m21 = L.add(b->m21_bytes);
+    const size_t o_pjobs = L.add(pjobs.size() * sizeof(plm::PairsJob));
+    const size_t o_units = L.add(units.size() * sizeof(int2));
     const size_t o_part = L.add(part_bytes);
     if ((st = b->ensure(L.total)) != PLM_OK) return st;
 
@@ -2801,6 +2881,21 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
         x.m21 = d_m21 + reinterpret_cast<uintptr_t>(x.m21);
         x.count = d_counts + reinterpret_cast<uintptr_t>(x.count);
     }
+    std::memset(&b->ptask, 0, sizeof(b->ptask));
+    if (umma) {
+        for (int j = 0, p = 0; j < n_jobs; ++j) {
+            if (task12[j] < 0) continue;
+            pjobs[p].part12 = tasks[task12[j]].part;
+            pjobs[p].part21 = best_lr ? tasks[task12[j] + 1].part : nullptr;
+            ++p;
+        }
+        b->ptask.q = d_arena + 2 * q_off;
+        b->ptask.arena = d_arena;
+        b->ptask.jobs = reinterpret_cast<const plm::PairsJob *>(D + o_pjobs);
+        b->ptask.units = reinterpret_cast<const int2 *>(D + o_units);
+        b->ptask.n1 = q_n;
+        b->ptask.n_units = static_cast<int>(units.size());
+    }
 
     // uploads: arenas straight from the caller's memory, tables through the pinned staging block
     const size_t tbl_bytes = L.total - b->o_tasks; // generous upper bound of the table region
@@ -2814,6 +2909,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
     const size_t s_merge = S.add(merge_map.size() * sizeof(int2));
     const size_t s_xjobs = S.add(xjobs.size() * sizeof(plm::XJob));
     const size_t s_xmap = S.add(xmap.size() * sizeof(int2));
+    const size_t s_pjobs = S.add(pjobs.size() * sizeof(plm::PairsJob));
+    const size_t s_units = S.add(units.size() * sizeof(int2));
     if ((st = ctx->ensure_pinned(S.total)) != PLM_OK) return st;
     char *H = ctx->h_buf;
     if (m12_arena) {
@@ -2827,6 +2924,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
     if (!merge_map.empty()) std::memcpy(H + s_merge, merge_map.data(), merge_map.size() * sizeof(int2));
     if (!xjobs.empty()) std::memcpy(H + s_xjobs, xjobs.data(), xjobs.size() * sizeof(plm::XJob));
     if (!xmap.empty()) std::memcpy(H + s_xmap, xmap.data(), xmap.size() * sizeof(int2));
+    if (!pjobs.empty()) std::memcpy(H + s_pjobs, pjobs.data(), pjobs.size() * sizeof(plm::PairsJob));
+    if (!units.empty()) std::memcpy(H + s_units, units.data(), units.size() * sizeof(int2));
     cudaStream_t s = ctx->stream;
     if (n_rows > 0 && !arena_dev) CU_TRY(cudaMemcpyAsync(D + o_arena, arena, size_t(n_rows) * 32, cudaMemcpyHostToDevice, s));
     if (m12_arena) {
@@ -2840,6 +2939,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
     if (!merge_map.empty()) CU_TRY(cudaMemcpyAsync(D + b->o_merge_map, H + s_merge, merge_map.size() * sizeof(int2), cudaMemcpyHostToDevice, s));
     if (!xjobs.empty()) CU_TRY(cudaMemcpyAsync(D + b->o_xjobs, H + s_xjobs, xjobs.size() * sizeof(plm::XJob), cudaMemcpyHostToDevice, s));
     if (!xmap.empty()) CU_TRY(cudaMemcpyAsync(D + b->o_xmap, H + s_xmap, xmap.size() * sizeof(int2), cudaMemcpyHostToDevice, s));
+    if (!pjobs.empty()) CU_TRY(cudaMemcpyAsync(D + o_pjobs, H + s_pjobs, pjobs.size() * sizeof(plm::PairsJob), cudaMemcpyHostToDevice, s));
+    if (!units.empty()) CU_TRY(cudaMemcpyAsync(D + o_units, H + s_units, units.size() * sizeof(int2), cudaMemcpyHostToDevice, s));
     CU_TRY(cudaStreamSynchronize(s)); // the pinned block is reused by the next call
 
     b->kind = 1;
@@ -2847,7 +2948,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
     b->n_m = n_m;
     b->nnr = nnr;
     b->best_lr = best_lr;
-    b->n_slice_ctas = static_cast<int>(cta_map.size());
+    b->n_slice_ctas = static_cast<int>(umma ? umma_ctas : static_cast<long long>(cta_map.size()));
+    b->n_umma_ctas = static_cast<int>(umma_ctas);
     b->n_merge_ctas = static_cast<int>(merge_map.size());
     b->n_x_ctas = static_cast<int>(xmap.size());
     b->h2d = static_cast<int64_t>((arena_dev ? 0 : size_t(n_rows) * 32) + S.total);
@@ -2983,7 +3085,18 @@ PLM_API int plm_batch_run(plm_batch *b) {
         // stages need no in-place transform (lower latency)
         (void)knn_variant_for(0); // reads PLM_KNN_VARIANT on first use
         const int forced = g_knn_variant;
-        if (forced == 0)
+        if (b->n_umma_ctas > 0) { // shared-query batch: both directions of every pair from one tensor-core product (K1c)
+            if ((st = umma_error_word(ctx)) != PLM_OK) return st;
+            if (!ctx->umma_pairs_attr_set) {
+                CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_pairs_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_PAIRS_SMEM));
+                CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_pairs_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_PAIRS_SMEM));
+                ctx->umma_pairs_attr_set = true;
+            }
+            if (b->best_lr)
+                plm::knn2_umma_pairs_kernel<true><<<b->n_umma_ctas, plm::KNN_UMMA_CTA_THREADS, plm::KNN_UMMA_PAIRS_SMEM, s>>>(b->ptask, ctx->umma_err_dev, g_peer_spin_ticks);
+            else
+                plm::knn2_umma_pairs_kernel<false><<<b->n_umma_ctas, plm::KNN_UMMA_CTA_THREADS, plm::KNN_UMMA_PAIRS_SMEM, s>>>(b->ptask, ctx->umma_err_dev, g_peer_spin_ticks);
+        } else if (forced == 0)
             plm::knn2_slice_list_kernel<BATCH_THREADS, 0><<<b->n_slice_ctas, BATCH_THREADS, 0, s>>>(tasks, reinterpret_cast<const int4 *>(D + b->o_cta_map));
         else if (forced == 1)
             plm::knn2_slice_list_kernel<BATCH_THREADS, 1><<<b->n_slice_ctas, BATCH_THREADS, 0, s>>>(tasks, reinterpret_cast<const int4 *>(D + b->o_cta_map));

@@ -485,6 +485,9 @@ class KeyframeDB:
     each pair with its own ratio tests and mutual check); here one query keyframe is matched against EVERY keyframe of
     the database in one batched launch (plm_batch_set_match_dev over the resident arena).  For several GPUs give every
     rank a contiguous range of keyframes: the pairs are independent, only the per-keyframe counts are gathered.
+    Every job of the batch shares the query slot, so with option "batch_umma" = 1 (read when the job tables are built
+    for a query size) both directions of every pair come from one int8 tensor-core product (DESIGN K1c); the results
+    are identical to the integer list kernels', which the automatic choice keeps (they measured faster).
 
     ``rows``: all descriptors of the database keyframes back to back (n x 32 uint8), ``kf_start``: n_kf + 1 row offsets;
     ``q_cap``: the largest query keyframe (rows reserved behind the database for the query slot)."""
