@@ -1,4 +1,6 @@
-// Brute-force Hamming top-2 on the tensor cores (knn2 variant 7, long scans only).
+// Brute-force Hamming top-2 on the tensor cores: the warp-specialised tcgen05 pipeline (umma_pipeline) and the
+// long-scan kernel built on it (knn2 variant 7, knn2_umma_kernel).  knn2_umma_pairs_kernel (plm_knn2_umma_pairs.cuh)
+// is the other kernel on the same pipeline.
 //
 // Over K = 256 bits the Hamming distance is an exact integer dot product.  With the query as +-1 bytes and the train
 // row as 0/1 bytes:
@@ -8,10 +10,10 @@
 //
 // One CTA per SM, the whole 512-column tensor memory.  A CTA owns a contiguous range of the (query group, 128-row
 // unit) work list, so every SM gets the same number of units whatever the number of query groups; the range is cut
-// into segments, one per query group it touches, each scanned in increasing row order.  The CTA is warp-specialised,
+// into segments, one per query group it touches, each scanned in increasing unit order.  The CTA is warp-specialised,
 // its roles meet only on mbarriers (full/empty pairs, every wait bounded), so loading, expansion, MMA and readout of
 // different units overlap:
-//   * producer (warp 12, one thread): packed train units (4 KB, rows * 32 B for a short last unit) -> a
+//   * producer (warp 12, one thread): packed train units (4 KB, rows * 32 B for a short unit) -> a
 //     KNN_UMMA_STAGES-deep ring with cp.async.bulk, completion counted in bytes on the stage's full barrier;
 //   * expanders (warps 8-11, thread = train row): packed stage -> 0/1 bytes in one of KNN_UMMA_BSTAGES B tiles,
 //     fence.proxy.async, arrive on the B tile's full barrier;
@@ -20,14 +22,17 @@
 //   * readout (warps 0-7, thread t = query t of the group = TMEM lane t & 127 of M-tile t >> 7): per segment the
 //     256 queries are expanded once to +-1 bytes (A = 2 M-tiles x 128 rows x 256 B, resident) and released to the
 //     MMA issuer on the A barrier; per unit all 128 accumulator columns are loaded, the buffer is released, and the
-//     blocked top-2 test of variants 2/3 runs on the registers (16 columns at a time, exact because columns are rows
-//     in increasing order).
+//     blocked top-2 test of variants 2/3 runs on the registers (16 columns at a time, exact because the columns of a
+//     unit are rows in increasing order and the test is strict).
 // A segment switch drains the pipeline once: the readout finishes the segment's last unit (so no MMA reads A any
 // more), writes its partials, rewrites A and arrives on the A barrier.
 // Operands are K-major with the 128-byte swizzle: a 256-byte row is two swizzle atoms along K, each operand tile is
 // [K half][rows][128 B] with 16-byte chunk c of row r stored at chunk c ^ (r & 7).
-// part[p][query] holds the (best, second) keys of segment p of the query's group; slots no CTA scanned are written
-// absent, so knn2_merge_kernel reads n_workers slots per query as for the integer kernels.
+//
+// knn2_umma_kernel: unit u is train rows [128 u, 128 u + 128) of one task, keys carry idx_base + row, and the
+// per-query second-best bound gthr is shared with the other CTAs.  part[p][query] holds the (best, second) keys of
+// segment p of the query's group; slots no CTA scanned are written absent, so knn2_merge_kernel reads n_workers slots
+// per query as for the integer kernels.
 #pragma once
 #include "plm_common.cuh"
 #include "plm_knn2.cuh"
@@ -40,10 +45,10 @@ constexpr int KNN_UMMA_ROWS = 128;                         // train rows per uni
 constexpr int KNN_UMMA_STAGES = 8;                         // packed-unit ring depth
 constexpr int KNN_UMMA_BSTAGES = 3;                        // expanded B tiles
 constexpr int KNN_UMMA_TILE_BYTES = 128 * 256;             // one 128-row operand tile of 256 int8 columns
-constexpr int KNN_UMMA_SMEM = 2 * KNN_UMMA_TILE_BYTES      // A (queries)
-                              + KNN_UMMA_BSTAGES * KNN_UMMA_TILE_BYTES // B ring
-                              + KNN_UMMA_STAGES * KNN_UMMA_ROWS * 32   // packed ring
-                              + 1024;                      // alignment of the swizzled tiles
+constexpr int KNN_UMMA_PIPE_BYTES = 2 * KNN_UMMA_TILE_BYTES // A (queries)
+                                    + KNN_UMMA_BSTAGES * KNN_UMMA_TILE_BYTES // B ring
+                                    + KNN_UMMA_STAGES * KNN_UMMA_ROWS * 32;  // packed ring
+constexpr int KNN_UMMA_SMEM = KNN_UMMA_PIPE_BYTES + 1024;  // + alignment of the swizzled tiles
 // rate kernel: A, B of up to 256 rows, and a 32 KB store target for the concurrent-store case
 constexpr int KNN_UMMA_RATE_SMEM = 4 * KNN_UMMA_TILE_BYTES + 1024;
 constexpr int KNN_UMMA_BLOCK = 16;                         // columns per blocked threshold test
@@ -69,11 +74,28 @@ __device__ __forceinline__ void umma_commit(uint32_t mbar) {
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// __syncthreads ordered against the tensor-core operations (TMEM alloc, MMA, loads) on both sides of it
+__device__ __forceinline__ void tc_syncthreads() { tc_fence_before(); __syncthreads(); tc_fence_after(); }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+// Warp-wide: COLS columns of tensor memory (a power of two >= 32), their address to *slot; the CTA then gives up its
+// allocation permit (it allocates once).
+template <int COLS>
+__device__ __forceinline__ void tmem_alloc(uint32_t *slot) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
+                 ::"r"(static_cast<uint32_t>(__cvta_generic_to_shared(slot))), "n"(COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+template <int COLS>
+__device__ __forceinline__ void tmem_dealloc(uint32_t tmem) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(COLS) : "memory");
+}
 
 __device__ __forceinline__ void mbar_init(uint32_t mbar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(mbar), "r"(count) : "memory");
 }
+// after the last mbar_init: the initialised barriers are visible to the other threads and the async proxy
+__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 // Bounded wait for the phase with the given parity; false after `limit` clock64 ticks.
 __device__ __forceinline__ bool mbar_wait(uint32_t mbar, uint32_t parity, long long limit) {
     const long long t0 = clock64();
@@ -146,6 +168,22 @@ __device__ __forceinline__ void expand_half(uint8_t *tile, int row, int half, co
 __host__ __device__ __forceinline__ long long umma_cta_of(long long x, long long total, long long ctas) {
     return ((x + 1) * ctas - 1) / total;
 }
+// Number of CTAs the items [first, first + n) of that list are spread over (n >= 1): the partial slots they need.
+__host__ __device__ __forceinline__ long long umma_ctas_spanned(long long first, long long n, long long total, long long ctas) {
+    return umma_cta_of(first + n - 1, total, ctas) - umma_cta_of(first, total, ctas) + 1;
+}
+// This CTA's partial slot in a run of items that starts at item `first` of the list of n1 queries x n_units units: its
+// index among the CTAs the run is spread over.
+__device__ __forceinline__ int umma_slot(long long first, int n1, long long n_units) {
+    const long long total = static_cast<long long>((n1 + KNN_UMMA_THREADS - 1) / KNN_UMMA_THREADS) * n_units;
+    return static_cast<int>(blockIdx.x - umma_cta_of(first, total, gridDim.x));
+}
+
+// The kernel's dynamic shared memory, aligned to 1024 bytes for the swizzled tiles.
+__device__ __forceinline__ uint8_t *umma_smem() {
+    extern __shared__ uint8_t smem_raw[];
+    return smem_raw + ((1024 - (static_cast<uint32_t>(__cvta_generic_to_shared(smem_raw)) & 1023)) & 1023);
+}
 
 #ifdef PLM_UMMA_STAMPS
 // Debug builds only (PLM_BUILD_DEFINES=-DPLM_UMMA_STAMPS): per CTA and role (0 readout, 1 expander, 2 producer, 3 MMA
@@ -155,13 +193,35 @@ constexpr int KNN_UMMA_STAMP_CTAS = 160;
 __device__ long long g_umma_stamps[KNN_UMMA_STAMP_CTAS][4][3];
 #endif
 
-__global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(const KnnTask t, int32_t *err, long long spin_limit) {
-    extern __shared__ uint8_t smem_raw[];
+// A segment as the readout sees it: units [u0, u0 + n) of query group g; this thread is query qi (valid: qi < n1), |q| = qn.
+struct UmmaSeg {
+    long long u0;
+    int g, n, qi, qn;
+    bool valid;
+};
+// Columns of one unit as the readout sees them: `rows` live columns, column j has key index key0 + j.
+struct UmmaCols {
+    int rows;
+    uint32_t key0;
+};
+
+// The pipeline over this CTA's share of the (query group of 256 of the n1 `queries`, unit) list of n_units units per
+// group; launched with KNN_UMMA_CTA_THREADS threads, one CTA per SM, shared memory from KNN_UMMA_PIPE_BYTES on is the
+// Scan's.  The Scan supplies the unit source and the readout's rules (each call is inlined):
+//   const uint4 *unit_src(long long u, int &rows)     producer: unit u's packed rows in global memory and their count
+//   void begin_segment(const UmmaSeg &s)              readout, after A is written
+//   UmmaCols begin_unit(const UmmaSeg &s, int i, int &thr)  unit s.u0 + i, its accumulators ready; may lower thr
+//   int threshold(unsigned long long B1)              the insert bound after an insert into (B0, B1)
+//   void loaded(int (&v)[2][32], int half, uint32_t k)  accumulator columns 64 half .. + 63 of buffer k, unmasked
+//   void end_unit(const UmmaSeg &s, int i, uint32_t k, int rows, unsigned long long &B0, unsigned long long &B1, int &thr)
+//   void end_segment(const UmmaSeg &s, unsigned long long B0, unsigned long long B1)
+template <class Scan>
+__device__ __forceinline__ void umma_pipeline(Scan &sc, const uint4 *queries, int n1, int n_units, int32_t *err, long long spin_limit) {
     // packed full / empty [STAGES], B full / empty [BSTAGES], accumulator full / empty [2], A ready
     __shared__ __align__(8) unsigned long long mbar[2 * KNN_UMMA_STAGES + 2 * KNN_UMMA_BSTAGES + 5];
     __shared__ uint32_t tmem_slot;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    uint8_t *smem = smem_raw + ((1024 - (static_cast<uint32_t>(__cvta_generic_to_shared(smem_raw)) & 1023)) & 1023); // 1024-aligned
+    uint8_t *smem = umma_smem();
     uint8_t *tileA = smem;                                  // 2 M-tiles
     uint8_t *tileB = smem + 2 * KNN_UMMA_TILE_BYTES;        // BSTAGES unit tiles
     const uint4 *ring = reinterpret_cast<const uint4 *>(smem + (2 + KNN_UMMA_BSTAGES) * KNN_UMMA_TILE_BYTES);
@@ -172,11 +232,7 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
     const uint32_t BFULL = PEMPTY + 8 * KNN_UMMA_STAGES, BEMPTY = BFULL + 8 * KNN_UMMA_BSTAGES;
     const uint32_t AFULL = BEMPTY + 8 * KNN_UMMA_BSTAGES, AEMPTY = AFULL + 16, AREADY = AEMPTY + 16;
 
-    if (warp == 0) {
-        const uint32_t slot = static_cast<uint32_t>(__cvta_generic_to_shared(&tmem_slot));
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(slot) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 0) tmem_alloc<512>(&tmem_slot);
     if (tid == 0) {
         for (int s = 0; s < KNN_UMMA_STAGES; ++s) {
             mbar_init(PFULL + 8 * s, 1);     // the producer's arrive + the copy's bytes
@@ -191,15 +247,12 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
             mbar_init(AEMPTY + 8 * k, KNN_UMMA_THREADS); // every readout thread
         }
         mbar_init(AREADY, KNN_UMMA_THREADS);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
+    tc_syncthreads();
     const uint32_t tmem = tmem_slot;
 
-    const int n1 = t.n1, nw = t.n_workers;
-    const long long n_units = t.n_units, groups = (n1 + KNN_UMMA_THREADS - 1) / KNN_UMMA_THREADS;
+    const long long groups = (n1 + KNN_UMMA_THREADS - 1) / KNN_UMMA_THREADS;
     const long long total = groups * n_units, ctas = gridDim.x;
     const long long x0 = static_cast<long long>(blockIdx.x) * total / ctas, x1 = (static_cast<long long>(blockIdx.x) + 1) * total / ctas;
     bool ok = true; // false after a wait timed out: this thread waits no more
@@ -225,7 +278,6 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
         u0 = x - static_cast<long long>(g) * n_units;
         n = static_cast<int>(min(x1, static_cast<long long>(g + 1) * n_units) - x);
     };
-    auto rows_of = [&](long long u) { return static_cast<int>(min(static_cast<long long>(KNN_UMMA_ROWS), t.n2 - u * KNN_UMMA_ROWS)); };
 
     if (warp == 12) { // producer: packed units -> ring
         if (lane == 0) {
@@ -238,9 +290,11 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
                 x += n;
                 for (int i = 0; i < n; ++i) {
                     wait(PEMPTY + 8 * s, ph ^ 1);
-                    const uint32_t bytes = static_cast<uint32_t>(rows_of(u0 + i)) * 32;
+                    int rows;
+                    const uint4 *src = sc.unit_src(u0 + i, rows);
+                    const uint32_t bytes = static_cast<uint32_t>(rows) * 32;
                     mbar_arrive_tx(PFULL + 8 * s, bytes);
-                    bulk_copy_g2s(sRing + s * (KNN_UMMA_ROWS * 32), t.db + 2 * ((u0 + i) * KNN_UMMA_ROWS), bytes, PFULL + 8 * s);
+                    bulk_copy_g2s(sRing + s * (KNN_UMMA_ROWS * 32), src, bytes, PFULL + 8 * s);
                     if (++s == KNN_UMMA_STAGES) { s = 0; ph ^= 1; }
 #ifdef PLM_UMMA_STAMPS
                     ++units_done;
@@ -248,7 +302,7 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
                 }
             }
         }
-    } else if (warp >= 8 && warp < 12) { // expanders: packed stage -> 0/1 bytes in a B tile (rows past n2: stale bits, masked later)
+    } else if (warp >= 8 && warp < 12) { // expanders: packed stage -> 0/1 bytes in a B tile (rows past the unit: stale bits, masked later)
         const int r = tid - KNN_UMMA_THREADS;
         int s = 0, j = 0;
         uint32_t ph = 0, bph = 0;
@@ -308,14 +362,11 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
     } else { // readout: thread = query of the group
         // this thread's accumulator lane: M-tile warp >> 2 at columns (warp >> 2) * 128, lanes 32 (warp & 3) ..
         const uint32_t tlane = tmem + (static_cast<uint32_t>(32 * (warp & 3)) << 16) + static_cast<uint32_t>((warp >> 2) * 128);
-        const uint32_t idx_base = static_cast<uint32_t>(t.idx_base); // idx_base + n2 <= 2^32 (checked by the host)
         uint32_t c = 0;
         for (long long x = x0; x < x1;) {
             int g, n;
             long long u0;
             segment(x, g, u0, n);
-            const int slot = static_cast<int>(blockIdx.x - umma_cta_of(static_cast<long long>(g) * n_units, total, ctas));
-            const bool last_of_group = x + n == static_cast<long long>(g + 1) * n_units;
             x += n;
 
             // queries of the group -> A (+-1 bytes), |q| per thread.  The previous segment's last accumulator wait
@@ -324,8 +375,8 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
             const bool valid = qi < n1;
             uint4 qlo = make_uint4(0, 0, 0, 0), qhi = qlo;
             if (valid) {
-                qlo = __ldg(t.q + 2 * static_cast<long long>(qi));
-                qhi = __ldg(t.q + 2 * static_cast<long long>(qi) + 1);
+                qlo = __ldg(queries + 2 * static_cast<long long>(qi));
+                qhi = __ldg(queries + 2 * static_cast<long long>(qi) + 1);
             }
             const int qn = __popc(qlo.x) + __popc(qlo.y) + __popc(qlo.z) + __popc(qlo.w) + __popc(qhi.x) + __popc(qhi.y) +
                            __popc(qhi.z) + __popc(qhi.w);
@@ -340,26 +391,16 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
             }
             fence_proxy_async_smem();
             mbar_arrive(AREADY);
+            const UmmaSeg sg{u0, g, n, qi, qn, valid};
+            sc.begin_segment(sg);
 
             unsigned long long B0 = KEY64_ABSENT, B1 = KEY64_ABSENT;
-            int thr = valid ? 1023 : 0, gcap = 1023; // a distance must be < thr to enter the top-2 (> 256: none yet)
-            uint32_t *gthr = (t.gthr && valid) ? t.gthr + qi : nullptr;
-            auto lower_thr = [&]() {
-                const int own = (B1 == KEY64_ABSENT) ? 1023 : static_cast<int>(B1 >> 32);
-                if (gthr && own < 1023) atomicMin(gthr, static_cast<uint32_t>(own));
-                thr = min(own, gcap);
-            };
+            int thr = valid ? 1023 : 0; // a distance must be < thr to enter the top-2 (> 256: none yet)
             for (int i = 0; i < n; ++i, ++c) {
                 const uint32_t k = c & 1u;
                 wait(AFULL + 8 * k, (c >> 1) & 1u);
                 tc_fence_after();
-                if (gthr) { // once per unit: the bound the other CTAs have reached (rows AT the bound stay in)
-                    const uint32_t gv = *reinterpret_cast<volatile uint32_t *>(gthr);
-                    gcap = static_cast<int>(min(gv, 1022u)) + 1;
-                    thr = min(thr, gcap);
-                }
-                const int rows = rows_of(u0 + i);
-                const uint32_t gbase = idx_base + static_cast<uint32_t>((u0 + i) * KNN_UMMA_ROWS);
+                const UmmaCols u = sc.begin_unit(sg, i, thr);
                 // two halves of 64 columns (128 live values would spill); the buffer is released for unit c + 2 as soon
                 // as the second half is in registers
 #pragma unroll
@@ -373,12 +414,13 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
                         tc_fence_before();
                         mbar_arrive(AEMPTY + 8 * k);
                     }
-                    if (rows < KNN_UMMA_ROWS) {
+                    sc.loaded(v, half, k);
+                    if (u.rows < KNN_UMMA_ROWS) {
 #pragma unroll
                         for (int q = 0; q < 2; ++q)
 #pragma unroll
                             for (int jj = 0; jj < 32; ++jj)
-                                if (64 * half + 32 * q + jj >= rows) v[q][jj] = 0x3FFFFFFF; // rows past n2: never below any bound
+                                if (64 * half + 32 * q + jj >= u.rows) v[q][jj] = 0x3FFFFFFF; // rows past the unit: never below any bound
                     }
 #pragma unroll
                     for (int q = 0; q < 2; ++q)
@@ -392,21 +434,18 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
 #pragma unroll
                                 for (int jj = 0; jj < KNN_UMMA_BLOCK; ++jj) {
                                     const int col = 64 * half + 32 * q + h + jj;
-                                    if (col < rows) top2_insert(B0, B1, make_key64(static_cast<uint32_t>(qn + v[q][h + jj]), gbase + col));
+                                    if (col < u.rows) top2_insert(B0, B1, make_key64(static_cast<uint32_t>(qn + v[q][h + jj]), u.key0 + col));
                                 }
-                                lower_thr();
+                                thr = sc.threshold(B1);
                             }
                         }
                 }
+                sc.end_unit(sg, i, k, u.rows, B0, B1, thr);
 #ifdef PLM_UMMA_STAMPS
                 ++units_done;
 #endif
             }
-            if (valid) {
-                t.part[static_cast<size_t>(slot) * n1 + qi] = make_ulonglong2(B0, B1);
-                if (last_of_group)
-                    for (int p = slot + 1; p < nw; ++p) t.part[static_cast<size_t>(p) * n1 + qi] = make_ulonglong2(KEY64_ABSENT, KEY64_ABSENT);
-            }
+            sc.end_segment(sg, B0, B1);
         }
     }
 #ifdef PLM_UMMA_STAMPS
@@ -417,10 +456,56 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
         g_umma_stamps[blockIdx.x][role][2] = units_done;
     }
 #endif
-    tc_fence_before();
-    __syncthreads(); // every MMA was waited for by the readout (or a wait timed out and the results are discarded)
-    tc_fence_after();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
+    tc_syncthreads(); // every MMA was waited for by the readout (or a wait timed out and the results are discarded)
+    if (warp == 0) tmem_dealloc<512>(tmem);
+}
+
+// knn2_umma_kernel's units and readout: rows of one task, keys idx_base + row, the shared bound gthr, one partial slot
+// per segment.
+struct KnnScan {
+    KnnTask t;
+    // per segment
+    int slot, gcap;
+    uint32_t *gthr;
+
+    __device__ __forceinline__ int rows_of(long long u) const { return static_cast<int>(min(static_cast<long long>(KNN_UMMA_ROWS), t.n2 - u * KNN_UMMA_ROWS)); }
+    __device__ __forceinline__ const uint4 *unit_src(long long u, int &rows) const {
+        rows = rows_of(u);
+        return t.db + 2 * (u * KNN_UMMA_ROWS);
+    }
+    __device__ __forceinline__ void begin_segment(const UmmaSeg &s) {
+        slot = umma_slot(static_cast<long long>(s.g) * t.n_units, t.n1, t.n_units);
+        gthr = (t.gthr && s.valid) ? t.gthr + s.qi : nullptr;
+        gcap = 1023;
+    }
+    __device__ __forceinline__ UmmaCols begin_unit(const UmmaSeg &s, int i, int &thr) {
+        if (gthr) { // once per unit: the bound the other CTAs have reached (rows AT the bound stay in)
+            const uint32_t gv = *reinterpret_cast<volatile uint32_t *>(gthr);
+            gcap = static_cast<int>(min(gv, 1022u)) + 1;
+            thr = min(thr, gcap);
+        }
+        // idx_base + n2 <= 2^32 (checked by the host)
+        const long long u = s.u0 + i;
+        return {rows_of(u), static_cast<uint32_t>(t.idx_base) + static_cast<uint32_t>(u * KNN_UMMA_ROWS)};
+    }
+    __device__ __forceinline__ int threshold(unsigned long long B1) const {
+        const int own = (B1 == KEY64_ABSENT) ? 1023 : static_cast<int>(B1 >> 32);
+        if (gthr && own < 1023) atomicMin(gthr, static_cast<uint32_t>(own));
+        return min(own, gcap);
+    }
+    __device__ __forceinline__ void loaded(int (&)[2][32], int, uint32_t) {}
+    __device__ __forceinline__ void end_unit(const UmmaSeg &, int, uint32_t, int, unsigned long long &, unsigned long long &, int &) {}
+    __device__ __forceinline__ void end_segment(const UmmaSeg &s, unsigned long long B0, unsigned long long B1) {
+        if (!s.valid) return;
+        t.part[static_cast<size_t>(slot) * t.n1 + s.qi] = make_ulonglong2(B0, B1);
+        if (s.u0 + s.n == t.n_units) // the last segment of the group
+            for (int p = slot + 1; p < t.n_workers; ++p) t.part[static_cast<size_t>(p) * t.n1 + s.qi] = make_ulonglong2(KEY64_ABSENT, KEY64_ABSENT);
+    }
+};
+
+__global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(const KnnTask t, int32_t *err, long long spin_limit) {
+    KnnScan sc{t};
+    umma_pipeline(sc, t.q, t.n1, t.n_units, err, spin_limit);
 }
 
 // Back-to-back 128 x N x 32 int8 MMAs on zeroed operands (one CTA per SM): the INT8 tensor-core rate of this card at
@@ -429,26 +514,19 @@ __global__ void __launch_bounds__(KNN_UMMA_CTA_THREADS, 1) knn2_umma_kernel(cons
 // KNN_UMMA_RATE_SMEM.
 template <int N, bool STS>
 __global__ void __launch_bounds__(128, 1) mma_i8_rate_kernel(int iters, int32_t *err, long long spin_limit) {
-    extern __shared__ uint8_t smem_raw[];
     __shared__ __align__(8) unsigned long long bar;
     __shared__ uint32_t tmem_slot;
-    uint8_t *smem = smem_raw + ((1024 - (static_cast<uint32_t>(__cvta_generic_to_shared(smem_raw)) & 1023)) & 1023); // 1024-aligned
+    uint8_t *smem = umma_smem();
     for (int i = threadIdx.x; i < 3 * KNN_UMMA_TILE_BYTES / 16; i += blockDim.x) reinterpret_cast<uint4 *>(smem)[i] = make_uint4(0, 0, 0, 0);
     const uint32_t sA = static_cast<uint32_t>(__cvta_generic_to_shared(smem)), sB = sA + KNN_UMMA_TILE_BYTES;
     const uint32_t sbar = static_cast<uint32_t>(__cvta_generic_to_shared(&bar));
-    if (threadIdx.x < 32) {
-        const uint32_t slot = static_cast<uint32_t>(__cvta_generic_to_shared(&tmem_slot));
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 256;" ::"r"(slot) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (threadIdx.x < 32) tmem_alloc<256>(&tmem_slot);
     if (threadIdx.x == 0) {
         mbar_init(sbar, 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     fence_proxy_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
+    tc_syncthreads();
     const uint32_t tmem = tmem_slot;
     // B is read as N rows from the zeroed tiles behind A
     constexpr uint32_t idesc = (KNN_UMMA_IDESC & ~(0x3Fu << 17)) | (uint32_t(N >> 3) << 17);
@@ -476,10 +554,8 @@ __global__ void __launch_bounds__(128, 1) mma_i8_rate_kernel(int iters, int32_t 
             if (clock64() - t0 > spin_limit) break;
         }
     }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 256;" ::"r"(tmem) : "memory");
+    tc_syncthreads();
+    if (threadIdx.x < 32) tmem_dealloc<256>(tmem);
 }
 
 } // namespace plm

@@ -83,9 +83,8 @@ struct plm_ctx {
     bool fused_attr_set = false;
     bool cluster_attr_set = false;
     int knn_occ[2][7] = {{0, 0, 0, 0, 0, 0, 0}, {0, 0, 0, 0, 0, 0, 0}};
-    bool umma_attr_set = false;
-    bool umma_pairs_attr_set = false;
-    // set by knn2_umma_kernel / mma_i8_rate_kernel when an MMA completion wait timed out (mapped pinned word)
+    bool umma_attr_set = false; // dynamic shared memory of knn2_umma_kernel and knn2_umma_pairs_kernel
+    // set by the tensor-core kernels when an MMA completion wait timed out (mapped pinned word)
     int32_t *umma_err_host = nullptr, *umma_err_dev = nullptr;
     size_t chunked_attr[2] = {0, 0};
     bool rows_attr_set = false;
@@ -314,6 +313,16 @@ int knn_ctas_per_sm(plm_ctx *ctx, int threads, int variant) {
     return cached;
 }
 
+// The (query group, unit) list of a tensor-core launch (knn2_umma_kernel, knn2_umma_pairs_kernel) and its grid: one
+// CTA per SM, at most one per item.
+struct UmmaGrid {
+    long long total, ctas;
+};
+UmmaGrid umma_grid(const plm_ctx *ctx, long long groups, long long units) {
+    const long long total = groups * units;
+    return {total, std::min<long long>(ctx->sm_count, total)};
+}
+
 // The train set is cut into units of <= 256 rows (one shared-memory stage) dealt round-robin to as many
 // workers per query block as fit on the chip at once: one wave of co-resident CTAs, no last-wave tail,
 // W partials per query.  Frame-sized problems get narrow CTAs and small units so that a single call
@@ -326,12 +335,11 @@ KnnPlan plan_knn(plm_ctx *ctx, int n1, long long n2, bool allow_two = false) {
         p.threads = p.qpb = plm::KNN_UMMA_THREADS;
         p.unit_rows = plm::KNN_UMMA_ROWS;
         const long long groups = std::max(1, (n1 + p.qpb - 1) / p.qpb), units = (n2 + p.unit_rows - 1) / p.unit_rows;
-        const long long total = groups * units, ctas = std::min<long long>(ctx->sm_count, total);
+        const UmmaGrid grid = umma_grid(ctx, groups, units);
         p.n_units = static_cast<int>(units);
         p.n_workers = 1;
         for (long long g = 0; g < groups; ++g)
-            p.n_workers = static_cast<int>(std::max<long long>(p.n_workers, plm::umma_cta_of(g * units + units - 1, total, ctas) -
-                                                                                  plm::umma_cta_of(g * units, total, ctas) + 1));
+            p.n_workers = static_cast<int>(std::max<long long>(p.n_workers, plm::umma_ctas_spanned(g * units, units, grid.total, grid.ctas)));
         p.share_thr = true;
         return p;
     }
@@ -382,6 +390,20 @@ int umma_error_word(plm_ctx *ctx) {
     return PLM_OK;
 }
 
+// Before a launch of knn2_umma_kernel or knn2_umma_pairs_kernel: the error word, and once per context their dynamic
+// shared memory.
+int umma_prepare(plm_ctx *ctx) {
+    const int st = umma_error_word(ctx);
+    if (st != PLM_OK) return st;
+    if (!ctx->umma_attr_set) {
+        CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_SMEM));
+        CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_pairs_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_PAIRS_SMEM));
+        CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_pairs_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_PAIRS_SMEM));
+        ctx->umma_attr_set = true;
+    }
+    return PLM_OK;
+}
+
 int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threads) {
     long long total = 0;
     for (int i = 0; i < n_tasks; ++i) {
@@ -394,8 +416,7 @@ int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threa
     // planned for the tensor-core kernel (plan_knn: single task, 256 queries per CTA)
     const bool umma = n_tasks == 1 && threads == plm::KNN_UMMA_THREADS;
     if (umma) {
-        const long long units = tp.t[0].n_units, groups = (tp.t[0].n1 + threads - 1) / threads;
-        total = std::min<long long>(ctx->sm_count, groups * units);
+        total = umma_grid(ctx, (tp.t[0].n1 + threads - 1) / threads, tp.t[0].n_units).ctas;
         tp.cta_split = static_cast<int>(total);
     }
     if (total == 0) return PLM_OK;
@@ -414,11 +435,7 @@ int launch_knn_slices(plm_ctx *ctx, plm::KnnTaskPair &tp, int n_tasks, int threa
     }
     if (n_tasks == 1 && tp.t[0].threads == 2 * threads) variant = 6; // planned with two queries per thread
     if (umma) {
-        if (!ctx->umma_attr_set) {
-            CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_SMEM));
-            ctx->umma_attr_set = true;
-        }
-        const int st = umma_error_word(ctx);
+        const int st = umma_prepare(ctx);
         if (st != PLM_OK) return st;
     }
     if (umma || (variant >= 2 && g_knn_fill)) {
@@ -2759,8 +2776,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
         for (int j = 0; j < n_jobs; ++j)
             if (!(jobs[j].n2 < 2 || (best_lr && jobs[j].n1 < 2))) n_units += (jobs[j].n2 + plm::KNN_UMMA_ROWS - 1) / plm::KNN_UMMA_ROWS;
         if (n_units > INT_MAX / 2) return fail(PLM_E_UNSUPPORTED, "batch too large for the tensor-core path");
-        const long long total = groups * n_units;
-        umma_ctas = std::min<long long>(ctx->sm_count, total);
+        const UmmaGrid grid = umma_grid(ctx, groups, n_units);
+        umma_ctas = grid.ctas;
         units.reserve(static_cast<size_t>(n_units));
         for (int j = 0; j < n_jobs; ++j) {
             const plm_pair_job &jb = jobs[j];
@@ -2774,10 +2791,8 @@ int batch_set_match_impl(plm_batch *b, const uint8_t *arena, const void *arena_d
             for (int u = 0; u < p.n_units; ++u) units.push_back(make_int2(static_cast<int>(pjobs.size()), u * plm::KNN_UMMA_ROWS));
             // slots of the 12 task: the most CTAs one (group, job) run is spread over (the kernel writes the unused ones)
             p.n_slots12 = 1;
-            for (long long g = 0; g < groups; ++g) {
-                const long long first = g * n_units + p.unit0, last = first + p.n_units - 1;
-                p.n_slots12 = static_cast<int>(std::max<long long>(p.n_slots12, plm::umma_cta_of(last, total, umma_ctas) - plm::umma_cta_of(first, total, umma_ctas) + 1));
-            }
+            for (long long g = 0; g < groups; ++g)
+                p.n_slots12 = static_cast<int>(std::max<long long>(p.n_slots12, plm::umma_ctas_spanned(g * n_units + p.unit0, p.n_units, grid.total, grid.ctas)));
             slots12[j] = p.n_slots12;
             pjobs.push_back(p);
         }
@@ -3086,12 +3101,7 @@ PLM_API int plm_batch_run(plm_batch *b) {
         (void)knn_variant_for(0); // reads PLM_KNN_VARIANT on first use
         const int forced = g_knn_variant;
         if (b->n_umma_ctas > 0) { // shared-query batch: both directions of every pair from one tensor-core product (K1c)
-            if ((st = umma_error_word(ctx)) != PLM_OK) return st;
-            if (!ctx->umma_pairs_attr_set) {
-                CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_pairs_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_PAIRS_SMEM));
-                CU_TRY(cudaFuncSetAttribute(plm::knn2_umma_pairs_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, plm::KNN_UMMA_PAIRS_SMEM));
-                ctx->umma_pairs_attr_set = true;
-            }
+            if ((st = umma_prepare(ctx)) != PLM_OK) return st;
             if (b->best_lr)
                 plm::knn2_umma_pairs_kernel<true><<<b->n_umma_ctas, plm::KNN_UMMA_CTA_THREADS, plm::KNN_UMMA_PAIRS_SMEM, s>>>(b->ptask, ctx->umma_err_dev, g_peer_spin_ticks);
             else
