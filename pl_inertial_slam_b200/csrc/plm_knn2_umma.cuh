@@ -16,7 +16,7 @@
 //   * producer (warp 12, one thread): packed train units (4 KB, rows * 32 B for a short unit) -> a
 //     KNN_UMMA_STAGES-deep ring with cp.async.bulk, completion counted in bytes on the stage's full barrier;
 //   * expanders (warps 8-11, thread = train row): packed stage -> 0/1 bytes in one of KNN_UMMA_BSTAGES B tiles,
-//     fence.proxy.async, arrive on the B tile's full barrier;
+//     fence.proxy.async, arrive on the B tile's full barrier and on the packed stage's empty barrier;
 //   * MMA issuer (warp 13, one thread): per unit 2 M-tiles x 8 K-steps of tcgen05.mma into accumulator buffer
 //     unit & 1, committed to the B tile's empty barrier and to the accumulator's full barrier;
 //   * readout (warps 0-7, thread t = query t of the group = TMEM lane t & 127 of M-tile t >> 7): per segment the
@@ -26,6 +26,9 @@
 //     unit are rows in increasing order and the test is strict).
 // A segment switch drains the pipeline once: the readout finishes the segment's last unit (so no MMA reads A any
 // more), writes its partials, rewrites A and arrives on the A barrier.
+// A stage is released only after its reads have completed: a packed stage after the expander has stored its values
+// into the B tile and fenced the proxies (its next writer is the async proxy), a B tile by the MMA commit, an
+// accumulator buffer after tcgen05.wait::ld, A at the segment's last accumulator wait.
 // Operands are K-major with the 128-byte swizzle: a 256-byte row is two swizzle atoms along K, each operand tile is
 // [K half][rows][128 B] with 16-byte chunk c of row r stored at chunk c ^ (r & 7).
 //
@@ -314,13 +317,18 @@ __device__ __forceinline__ void umma_pipeline(Scan &sc, const uint4 *queries, in
             for (int i = 0; i < n; ++i) {
                 wait(PFULL + 8 * s, ph);
                 const uint4 lo = ring[s * (2 * KNN_UMMA_ROWS) + 2 * r], hi = ring[s * (2 * KNN_UMMA_ROWS) + 2 * r + 1];
-                mbar_arrive(PEMPTY + 8 * s);
-                if (++s == KNN_UMMA_STAGES) { s = 0; ph ^= 1; }
                 wait(BEMPTY + 8 * j, bph ^ 1);
                 expand_half<false>(tileB + j * KNN_UMMA_TILE_BYTES, r, 0, lo);
                 expand_half<false>(tileB + j * KNN_UMMA_TILE_BYTES, r, 1, hi);
-                fence_proxy_async_smem(); // generic-proxy stores -> visible to the MMA (async proxy)
+                // One proxy fence orders this thread's generic-proxy accesses against the async proxy in both
+                // directions: the B-tile stores before the MMA reads them, and the packed-stage loads (complete: their
+                // values were just stored) before the producer's next cp.async.bulk writes that stage.  The mbarrier's
+                // release/acquire alone orders generic accesses only, and an arrive issued right after the loads does
+                // not wait for them: the stage could be refilled with unit c + KNN_UMMA_STAGES before they read it.
+                fence_proxy_async_smem();
                 mbar_arrive(BFULL + 8 * j);
+                mbar_arrive(PEMPTY + 8 * s);
+                if (++s == KNN_UMMA_STAGES) { s = 0; ph ^= 1; }
                 if (++j == KNN_UMMA_BSTAGES) { j = 0; bph ^= 1; }
 #ifdef PLM_UMMA_STAMPS
                 ++units_done;
