@@ -26,6 +26,8 @@
  *                           device-resident keyframes   src/mapHandler.cpp:3116-3237, 3325-3378
  *   plm_med_desc / plm_dev_med_desc   PLSLAM::MapPoint / MapLine::updateAverageDescDir (the producer of the
  *                           map's med_desc rows)           src/mapFeatures.cpp:51-93, 121-163
+ *   plm_localmap_*          resident local map: map_points / map_lines updated in place and matchMap2KFPoints / Lines
+ *                           from the resident rows         src/mapHandler.cpp:583-803, src/mapFeatures.cpp
  *
  * The C++ replacement of stvo-pl/src/matching.cpp that keeps the StVO:: signatures and calls this
  * ABI is pl_inertial_slam_b200/csrc/stvo_matching_gpu.cpp (see INTEGRATION.md).
@@ -650,6 +652,93 @@ int64_t plm_loopdb_size(const plm_loopdb *db);
  * rows in, the score row out). */
 int64_t plm_loopdb_h2d_bytes(const plm_loopdb *db);
 int64_t plm_loopdb_d2h_bytes(const plm_loopdb *db);
+
+/* ---- resident local map (MapHandler's map_points / map_lines + matchMap2KFPoints / Lines) ------------------------ */
+/* The landmarks of MapHandler's local-mapping thread, resident on the context's device: positions, the `active` byte of
+ * plm_map_select, med_desc / med_dir and every observation (descriptor + direction).  A landmark crosses PCIe once, when
+ * it is inserted; later calls send only what changes, and matchMap2KF* runs from the resident rows.  One store holds one
+ * kind (is_lines = 0: points, X = 3 doubles; 1: segments, X = 6 doubles), as the reference keeps map_points and
+ * map_lines apart.  A landmark's index (slot) is the reference's index into map_points / map_lines: slots are handed
+ * out in insertion order and never reused.  lm_capacity / obs_capacity: landmarks / observation rows the arenas are
+ * first sized for (0 = 1024 / 4096); every arena grows geometrically.  Each landmark owns a reserved run of
+ * observation rows (4 when inserted); a list that outgrows its run moves, device to device, to the tail of the arenas
+ * with twice the room.  One store may be used by one host thread at a time.
+ *
+ * Every call validates its arguments on the host before any device work (argument errors never touch the GPU); a failed
+ * call (argument error, invalid or culled slot, duplicate cull, PLM_E_UNSUPPORTED, allocation failure) leaves the store
+ * unchanged.  Cost per call, whatever the number of landmarks (n = entries of the call, u = distinct landmarks an
+ * observation call touches, n2 = keyframe features, c = grid cells, k = cell_start[c], per = 1 points / 2 segments):
+ *   insert            1 host -> device copy of n * (56 + 24 per) bytes, 1 launch
+ *   add_observations  1 host -> device copy of 60 n + 20 u bytes (rows, directions, destination rows; per landmark its
+ *                     old and new run), 3 launches (append + the two medoid kernels) and a memset
+ *   set_positions     1 host -> device copy of n * (4 + 24 per) bytes, 1 launch
+ *   set_active        1 host -> device copy of 5 n bytes, 1 launch
+ *   cull              1 host -> device copy of 4 n bytes, 1 launch
+ * An update call makes no device -> host copy and no synchronisation; it only waits for the host -> device copy of the
+ * previous update, whose pinned staging block it reuses.  The cost of plm_localmap_match_kf is stated with it. */
+typedef struct plm_localmap plm_localmap;
+int plm_localmap_create(plm_ctx *ctx, int is_lines, int lm_capacity, int64_t obs_capacity, plm_localmap **out);
+int plm_localmap_destroy(plm_localmap *lm);
+/* Appends n landmarks with the next slots (*first_idx = the first; may be NULL): X (n x 3 or n x 6 doubles), one
+ * observation each (desc: n x 32 bytes `step` apart, dir: n x 3 doubles), as the MapPoint / MapLine constructors
+ * (mapFeatures.cpp:29-40, :99-110): med_desc = desc, med_dir = dir.  New landmarks are active. */
+int plm_localmap_insert(plm_localmap *lm, int n, const double *X, const uint8_t *desc, size_t step, const double *dir,
+                        int *first_idx);
+/* Appends observation i (desc row i, dir row i) to landmark lm_idx[i], in array order (a landmark may appear several
+ * times), then recomputes med_desc and med_dir of every touched landmark in one batch of the medoid kernels
+ * (plm_med_desc): the result is updateAverageDescDir of the final list, i.e. what the reference leaves after its
+ * recompute per append. */
+int plm_localmap_add_observations(plm_localmap *lm, int n, const int32_t *lm_idx, const uint8_t *desc, size_t step,
+                                  const double *dir);
+/* X[idx[i]] = row i of X (e.g. after local bundle adjustment); active[idx[i]] = val[i].  A slot listed twice takes its
+ * last entry. */
+int plm_localmap_set_positions(plm_localmap *lm, int n, const int32_t *idx, const double *X);
+int plm_localmap_set_active(plm_localmap *lm, int n, const int32_t *idx, const uint8_t *val);
+/* map_points[idx[i]] = NULL: the slots are never selected again; setting, updating or reading a culled slot, or culling
+ * it again (also twice in one call), returns PLM_E_INVALID. */
+int plm_localmap_cull(plm_localmap *lm, int n, const int32_t *idx);
+/* The keyframe side of plm_localmap_match_kf, from the host: its still unmatched features (desc: n2 x 32 bytes `step`
+ * apart), their grid (CSR as plm_match_grid_points takes it: cell_start = grid_rows * grid_cols + 1 entries, cell_items =
+ * cell_start[last] entries), dirs2 (n2 x 2, segments only) and feat for the gate: pl (n2 x 2) for points, le (n2 x 3)
+ * for segments. */
+typedef struct plm_localmap_kf {
+    const uint8_t *desc;
+    size_t step;
+    const int32_t *cell_start;
+    const int32_t *cell_items;
+    const double *dirs2;
+    const double *feat;
+    int32_t n2, grid_rows, grid_cols, pad_;
+} plm_localmap_kf;
+/* The config values matchMap2KF* reads: ratio (matchGrid, Config::minRatio12P), line_sim_th (Config::lineSimTh), max_epip
+ * (SlamConfig::maxKFEpipP / L), nnr (the fallback's float ratio), ws (Config::matchingF2FWs: window +-ws),
+ * best_lr (Config::bestLRMatches), fast_matching (SlamConfig::fastMatching), min_matches (minPointMatches /
+ * minLineMatches). */
+typedef struct plm_localmap_params {
+    double ratio, line_sim_th, max_epip;
+    float nnr;
+    int32_t ws, best_lr, fast_matching, min_matches, pad_;
+} plm_localmap_params;
+/* MapHandler::matchMap2KFPoints / Lines (mapHandler.cpp:583-682, :685-803) from the resident rows in one call: selection
+ * (plm_map_select over every slot with its active byte), gather of med_desc of the selected rows, matchGrid with a +-ws
+ * window when fast_matching, then StVO::match(nnr) on the same vector (stale entries kept) when
+ * n_sel > min_matches && matches < min_matches -- n_sel standing for both feature counts, as the reference passes them
+ * -- and the reprojection gate.  Outputs: *n_sel selected slots in order (sel), m12 and ok per selected slot, *count =
+ * the reference's match count after the gate; sel / m12 / ok need room for plm_localmap_size entries.  An empty map,
+ * n_sel == 0 or n2 == 0 give m12 = -1, ok = 0, count 0.  Results equal plm_map_select + plm_match_grid_* + plm_match +
+ * plm_map_gate on the same rows bit for bit.  Synchronises at most three times: for n_sel (it sizes the grid launches),
+ * for the grid count (only when fast_matching and n_sel > min_matches) and at the end.  Host -> device: one copy of
+ * n2 * (48 + 24 is_lines) + 4 (c + 1 + k) bytes; device -> host: 4 + 9 n_sel + 4 bytes, + 4 with the grid count. */
+int plm_localmap_match_kf(plm_localmap *lm, const plm_map_view *v, const plm_localmap_kf *kf, const plm_localmap_params *p,
+                          int32_t *sel, int32_t *m12, uint8_t *ok, int *n_sel, int *count);
+/* Reads n slots back: X (n x 3 or 6), med_desc (n x 32 bytes), med_dir (n x 3), n_obs (observations per slot); each may
+ * be NULL.  One device -> host copy and one synchronisation. */
+int plm_localmap_read(plm_localmap *lm, int n, const int32_t *idx, double *X, uint8_t *med_desc, double *med_dir, int32_t *n_obs);
+/* Slots handed out (culled ones included). */
+int64_t plm_localmap_size(const plm_localmap *lm);
+/* Cumulative bytes copied host -> device / device -> host by every call (the formulas above; read-backs included). */
+int64_t plm_localmap_h2d_bytes(const plm_localmap *lm);
+int64_t plm_localmap_d2h_bytes(const plm_localmap *lm);
 
 /* Tuning knobs (measurement / A-B tests only; results never depend on them):
  *   "knn_variant"  -1 = automatic (default: 3 for train sets >= 65 536 rows, 5 for short train sides with >= 2^26 pairs,

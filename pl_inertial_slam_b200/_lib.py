@@ -48,6 +48,17 @@ class MapView(C.Structure):
                 ("inv_width", C.c_double), ("inv_height", C.c_double), ("width", C.c_int32), ("height", C.c_int32)]
 
 
+class LocalMapKf(C.Structure):
+    _fields_ = [("desc", vp), ("step", C.c_size_t), ("cell_start", vp), ("cell_items", vp), ("dirs2", vp), ("feat", vp),
+                ("n2", C.c_int32), ("grid_rows", C.c_int32), ("grid_cols", C.c_int32), ("pad_", C.c_int32)]
+
+
+class LocalMapParams(C.Structure):
+    _fields_ = [("ratio", C.c_double), ("line_sim_th", C.c_double), ("max_epip", C.c_double), ("nnr", C.c_float),
+                ("ws", C.c_int32), ("best_lr", C.c_int32), ("fast_matching", C.c_int32), ("min_matches", C.c_int32),
+                ("pad_", C.c_int32)]
+
+
 class PeerGroup(C.Structure):
     _fields_ = [("xchg", C.POINTER(vp)), ("gather", C.POINTER(vp)), ("rank", C.c_int32), ("world", C.c_int32),
                 ("q_cap", C.c_int32), ("pad_", C.c_int32), ("n_rows_cap", C.c_int64), ("xchg_epoch", C.c_uint32),
@@ -202,6 +213,19 @@ SIGNATURES = {
     "plm_loopdb_size": (C.c_int64, [vp]),
     "plm_loopdb_h2d_bytes": (C.c_int64, [vp]),
     "plm_loopdb_d2h_bytes": (C.c_int64, [vp]),
+    "plm_localmap_create": (C.c_int, [vp, C.c_int, C.c_int, C.c_int64, C.POINTER(vp)]),
+    "plm_localmap_destroy": (C.c_int, [vp]),
+    "plm_localmap_insert": (C.c_int, [vp, C.c_int, f64p, u8p, C.c_size_t, f64p, intp]),
+    "plm_localmap_add_observations": (C.c_int, [vp, C.c_int, i32p, u8p, C.c_size_t, f64p]),
+    "plm_localmap_set_positions": (C.c_int, [vp, C.c_int, i32p, f64p]),
+    "plm_localmap_set_active": (C.c_int, [vp, C.c_int, i32p, u8p]),
+    "plm_localmap_cull": (C.c_int, [vp, C.c_int, i32p]),
+    "plm_localmap_match_kf": (C.c_int, [vp, C.POINTER(MapView), C.POINTER(LocalMapKf), C.POINTER(LocalMapParams), i32p,
+                                        i32p, u8p, intp, intp]),
+    "plm_localmap_read": (C.c_int, [vp, C.c_int, i32p, f64p, u8p, f64p, i32p]),
+    "plm_localmap_size": (C.c_int64, [vp]),
+    "plm_localmap_h2d_bytes": (C.c_int64, [vp]),
+    "plm_localmap_d2h_bytes": (C.c_int64, [vp]),
     "plm_med_desc": (C.c_int, [vp, u8p, C.c_int64, C.c_size_t, f64p, i32p, C.c_int, i32p, u8p, f64p]),
     "plm_dev_med_desc": (C.c_int, [vp, vp, C.c_int64, vp, vp, C.c_int, vp, vp, vp, vp]),
     "plm_set_option": (C.c_int, [C.c_char_p, C.c_int]),

@@ -29,18 +29,41 @@ namespace plm {
 constexpr int MED_WARPS = 4;   // landmarks in flight per CTA of the warp kernel
 constexpr int MED_CTA_THREADS = 256;
 
+// A work item finds its list in one of two ways:
+//  * CSR (lm_ids == null): item l is landmark l, its rows are obs_start[l] .. obs_start[l+1]-1;
+//  * start / length table (lm_ids != null): item w is landmark l = lm_ids[w], its rows are obs_start[l] ..
+//    obs_start[l] + obs_len[l] - 1 (the reserved runs of the resident local map, plm_localmap_api.inl); med_desc and
+//    med_dir are then written at landmark l, med_idx at item w.
 struct MedArgs {
     const uint4 *desc;        // n_obs x 32 B
     const double *dirs;       // n_obs x 3, or null
-    const int32_t *obs_start; // n_lm + 1
+    const int32_t *obs_start; // n_lm + 1 (CSR) or one entry per landmark (table)
     long long n_obs;
-    int n_lm;
+    int n_lm;                 // work items
     int32_t *med_idx;        // n_lm: winning position inside the list, -1 for an empty / malformed list
     uint4 *med_desc;         // n_lm x 32 B, or null
     const int32_t *dst_rows; // optional: landmark l writes row dst_rows[l] of med_desc (< 0: skip) -- scatter into a map DB
     double *med_dir;         // n_lm x 3, or null
-    int32_t *work;           // [0] = number of long lists, [1 ..] = their landmark ids
+    int32_t *work;           // [0] = number of long lists, [1 ..] = their item ids
+    const int32_t *lm_ids;   // optional: landmark of each item (table form)
+    const int32_t *obs_len;  // table form: list length per landmark
 };
+
+// Rows of item w: [*lo, *lo + returned length) (the raw length; the caller rejects malformed ranges).
+template <bool TABLE>
+__device__ __forceinline__ long long med_list(const MedArgs &a, long long w, long long &lo) {
+    if (TABLE) {
+        const int l = __ldg(a.lm_ids + w);
+        lo = __ldg(a.obs_start + l);
+        return __ldg(a.obs_len + l);
+    }
+    lo = __ldg(a.obs_start + w);
+    return static_cast<long long>(__ldg(a.obs_start + w + 1)) - lo;
+}
+
+// Row of med_desc / med_dir that item w writes.
+template <bool TABLE>
+__device__ __forceinline__ long long med_out(const MedArgs &a, long long w) { return TABLE ? __ldg(a.lm_ids + w) : w; }
 
 // int(1 + 0.5 * (n - 1)) of mapFeatures.cpp:79 for n >= 2
 __device__ __forceinline__ int med_rank(int n) { return 1 + (n - 1) / 2; }
@@ -96,7 +119,7 @@ __device__ __forceinline__ void med_sort_network(int (&d)[32]) { PLM_SORT_NET_32
 // real entries (mapFeatures.cpp:79); the G - n unused slots hold 0x7FFF and sink to the end.  The classes are cut so
 // that r is one of G / 4 positions (lists of a 16- or 32-lane pass have n > G / 2), and only those outputs of the
 // network are read -- the compiler prunes the comparators that none of them depends on.
-template <int G>
+template <int G, bool TABLE>
 __device__ __forceinline__ void med_desc_pass(const MedArgs &a, double *sdir, long long lm, long long lo, int n, int nmax,
                                               bool valid) {
     const int lane = threadIdx.x & 31, sl = lane & (G - 1);
@@ -151,7 +174,7 @@ __device__ __forceinline__ void med_desc_pass(const MedArgs &a, double *sdir, lo
     if (valid) {
         if (sl == 0) a.med_idx[lm] = best;
         if (a.med_desc) {
-            const long long row = a.dst_rows ? __ldg(a.dst_rows + lm) : lm;
+            const long long row = a.dst_rows ? __ldg(a.dst_rows + lm) : med_out<TABLE>(a, lm);
             if (row >= 0 && sl == (best < 0 ? 0 : best)) { // the winner writes its own registers (zeros for an empty list)
                 a.med_desc[2 * row] = q.lo;
                 a.med_desc[2 * row + 1] = q.hi;
@@ -172,7 +195,7 @@ __device__ __forceinline__ void med_desc_pass(const MedArgs &a, double *sdir, lo
                     if (j < n) acc = __dadd_rn(acc, g[3 * j]);
                 r = __ddiv_rn(acc, static_cast<double>(n));
             }
-            a.med_dir[3 * lm + sl] = r;
+            a.med_dir[3 * med_out<TABLE>(a, lm) + sl] = r;
         }
         __syncwarp();
     }
@@ -191,6 +214,7 @@ __device__ __forceinline__ int med_nth_bit(unsigned m, int g) {
 // lanes for lists of <= 8 observations, 2 x 16 for <= 16, 1 x 32 for <= 32.  (Packing by the longest list of 4
 // NEIGHBOURS put 86 % of a Poisson(8) map into the 16-lane form.)  Longer lists go to the work list of
 // med_desc_cta_kernel.
+template <bool TABLE>
 __global__ void __launch_bounds__(32 * MED_WARPS) med_desc_warp_kernel(MedArgs a) {
     __shared__ double sdir_all[MED_WARPS][32 * 3];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -202,8 +226,7 @@ __global__ void __launch_bounds__(32 * MED_WARPS) med_desc_warp_kernel(MedArgs a
         lo = 0;
         n = -2; // past the end
         if (chunk < n_chunks && my_lm < a.n_lm) {
-            lo = __ldg(a.obs_start + my_lm);
-            const long long len = static_cast<long long>(__ldg(a.obs_start + my_lm + 1)) - lo;
+            const long long len = med_list<TABLE>(a, my_lm, lo);
             n = (lo < 0 || len < 0 || lo + len > a.n_obs) ? 0 : static_cast<int>(min(len, 1LL << 30)); // malformed: empty
         }
     };
@@ -215,8 +238,8 @@ __global__ void __launch_bounds__(32 * MED_WARPS) med_desc_warp_kernel(MedArgs a
         const long long my_lo = nx_lo;
         const int my_n = nx_n;
         // the chunk's observations are one contiguous range of the arenas: ask L2 for all of it now, the passes below
-        // then wait on L2, not on HBM
-        {
+        // then wait on L2, not on HBM (CSR form only: the runs of the table form are scattered)
+        if (!TABLE) {
             const long long first = __shfl_sync(0xFFFFFFFFu, my_lo, 0);
             const unsigned live = __ballot_sync(0xFFFFFFFFu, my_n >= 0);
             const int last_lane = 31 - __clz(live | 1u);
@@ -249,7 +272,7 @@ __global__ void __launch_bounds__(32 * MED_WARPS) med_desc_warp_kernel(MedArgs a
             const int n = src >= 0 ? n_src : 0;
             const long long lo = __shfl_sync(0xFFFFFFFFu, my_lo, src & 31);
             const int nmax = __reduce_max_sync(0xFFFFFFFFu, n);
-            med_desc_pass<8>(a, sdir, chunk * 32 + src, lo, n, nmax, src >= 0);
+            med_desc_pass<8, TABLE>(a, sdir, chunk * 32 + src, lo, n, nmax, src >= 0);
 #pragma unroll
             for (int t = 0; t < 4; ++t) m8 &= m8 - 1;
         }
@@ -259,7 +282,7 @@ __global__ void __launch_bounds__(32 * MED_WARPS) med_desc_warp_kernel(MedArgs a
             const int n = src >= 0 ? n_src : 0;
             const long long lo = __shfl_sync(0xFFFFFFFFu, my_lo, src & 31);
             const int nmax = __reduce_max_sync(0xFFFFFFFFu, n);
-            med_desc_pass<16>(a, sdir, chunk * 32 + src, lo, n, nmax, src >= 0);
+            med_desc_pass<16, TABLE>(a, sdir, chunk * 32 + src, lo, n, nmax, src >= 0);
             m16 &= m16 - 1;
             m16 &= m16 - 1;
         }
@@ -267,7 +290,7 @@ __global__ void __launch_bounds__(32 * MED_WARPS) med_desc_warp_kernel(MedArgs a
             const int src = __ffs(m32) - 1;
             const int n = __shfl_sync(0xFFFFFFFFu, my_n, src);
             const long long lo = __shfl_sync(0xFFFFFFFFu, my_lo, src);
-            med_desc_pass<32>(a, sdir, chunk * 32 + src, lo, n, n, true);
+            med_desc_pass<32, TABLE>(a, sdir, chunk * 32 + src, lo, n, n, true);
             m32 &= m32 - 1;
         }
     }
@@ -279,6 +302,7 @@ constexpr int MED_CTA_CACHE_N = 128; // lists up to this length keep their rows 
 // the rows are staged in shared memory, every pair is computed once into a uint16 matrix, and a row's rank search
 // (smallest v with #{d <= v} >= rank + 1, bisection over 0 .. 256) is shared by 2 or 4 lanes that each count a
 // strided part of the row and add up by shuffle; longer lists fall back to one thread per row recomputing distances.
+template <bool TABLE>
 __global__ void __launch_bounds__(MED_CTA_THREADS) med_desc_cta_kernel(MedArgs a) {
     __shared__ unsigned long long s_best;
     __shared__ uint16_t s_dist[MED_CTA_CACHE_N * MED_CTA_CACHE_N];
@@ -287,8 +311,8 @@ __global__ void __launch_bounds__(MED_CTA_THREADS) med_desc_cta_kernel(MedArgs a
     const int n_work = a.work[0];
     for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
         const long long lm = a.work[1 + w];
-        const long long lo = __ldg(a.obs_start + lm);
-        const int n = static_cast<int>(static_cast<long long>(__ldg(a.obs_start + lm + 1)) - lo);
+        long long lo;
+        const int n = static_cast<int>(med_list<TABLE>(a, lm, lo));
         if (threadIdx.x == 0) s_best = KEY64_ABSENT;
         const bool cached = n <= MED_CTA_CACHE_N;
         const int need = med_rank(n) + 1;
@@ -351,17 +375,18 @@ __global__ void __launch_bounds__(MED_CTA_THREADS) med_desc_cta_kernel(MedArgs a
         const int best = static_cast<int>(s_best & 0xFFFFFFFFull);
         if (threadIdx.x == 0) a.med_idx[lm] = best;
         if (a.med_desc && threadIdx.x < 2) {
-            const long long row = a.dst_rows ? __ldg(a.dst_rows + lm) : lm;
+            const long long row = a.dst_rows ? __ldg(a.dst_rows + lm) : med_out<TABLE>(a, lm);
             if (row >= 0) a.med_desc[2 * row + threadIdx.x] = __ldg(a.desc + 2 * (lo + best) + threadIdx.x);
         }
         if (a.med_dir && a.dirs && threadIdx.x >= 32 && threadIdx.x < 35) {
             const int c = threadIdx.x - 32;
+            const long long out = med_out<TABLE>(a, lm);
             if (cached) { // same sequential sum as med_dir_component, from the staged copy (60 dependent L2 reads otherwise)
                 double acc = 0.0;
                 for (int i = 0; i < n; ++i) acc = __dadd_rn(acc, s_dirs[3 * i + c]);
-                a.med_dir[3 * lm + c] = __ddiv_rn(acc, static_cast<double>(n));
+                a.med_dir[3 * out + c] = __ddiv_rn(acc, static_cast<double>(n));
             } else {
-                a.med_dir[3 * lm + c] = med_dir_component(a.dirs, lo, n, c);
+                a.med_dir[3 * out + c] = med_dir_component(a.dirs, lo, n, c);
             }
         }
         __syncthreads();

@@ -26,6 +26,7 @@
 #include "plm_knn2.cuh"
 #include "plm_knn2_umma.cuh"
 #include "plm_knn2_umma_pairs.cuh"
+#include "plm_localmap.cuh"
 #include "plm_map.cuh"
 #include "plm_reproj.cuh"
 #include "plm_micro.cuh"
@@ -1767,10 +1768,13 @@ int launch_med_desc(plm_ctx *ctx, plm::MedArgs a) {
     CU_TRY(cudaMemsetAsync(a.work, 0, 4, ctx->stream));
     const int per_cta = 32 * plm::MED_WARPS; // a warp takes a chunk of 32 landmarks at a time
     const int ctas = std::min((a.n_lm + per_cta - 1) / per_cta, ctx->sm_count * 32);
-    plm::med_desc_warp_kernel<<<ctas, 32 * plm::MED_WARPS, 0, ctx->stream>>>(a);
+    // the start / length-table form (resident local map) is its own instantiation: the CSR kernels stay as they were
+    if (a.lm_ids) plm::med_desc_warp_kernel<true><<<ctas, 32 * plm::MED_WARPS, 0, ctx->stream>>>(a);
+    else plm::med_desc_warp_kernel<false><<<ctas, 32 * plm::MED_WARPS, 0, ctx->stream>>>(a);
     ctx->launches++;
     CU_TRY(cudaGetLastError());
-    plm::med_desc_cta_kernel<<<ctx->sm_count * 2, plm::MED_CTA_THREADS, 0, ctx->stream>>>(a);
+    if (a.lm_ids) plm::med_desc_cta_kernel<true><<<ctx->sm_count * 2, plm::MED_CTA_THREADS, 0, ctx->stream>>>(a);
+    else plm::med_desc_cta_kernel<false><<<ctx->sm_count * 2, plm::MED_CTA_THREADS, 0, ctx->stream>>>(a);
     ctx->launches++;
     CU_TRY(cudaGetLastError());
     return PLM_OK;
@@ -3541,6 +3545,32 @@ PLM_API int plm_map_gate(plm_ctx *ctx, int is_lines, const double *pf, const int
     return PLM_OK;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Device arenas of the resident stores (plm_loopdb_*, plm_localmap_*): every arena grows geometrically
+namespace {
+
+// Replaces *buf (used_bytes of content) by a new allocation of new_bytes holding the same content.  On failure *buf is
+// unchanged.
+int arena_realloc(plm_ctx *ctx, void **buf, size_t used_bytes, size_t new_bytes) {
+    void *nb = nullptr;
+    CU_TRY(cudaMalloc(&nb, new_bytes));
+    cudaError_t e = cudaSuccess;
+    if (used_bytes) e = cudaMemcpyAsync(nb, *buf, used_bytes, cudaMemcpyDeviceToDevice, ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) {
+        cudaFree(nb);
+        return fail(PLM_E_CUDA, std::string("device arena growth: ") + cudaGetErrorString(e));
+    }
+    if (*buf) cudaFree(*buf);
+    *buf = nb;
+    return PLM_OK;
+}
+
+int64_t arena_grown(int64_t cap, int64_t need) { return std::max<int64_t>(need, cap * 2); }
+
+} // namespace
+
 #include "plm_frames_api.inl"
 #include "plm_shard_api.inl"
 #include "plm_loopdb_api.inl"
+#include "plm_localmap_api.inl"
