@@ -23,7 +23,8 @@
 //     256 queries are expanded once to +-1 bytes (A = 2 M-tiles x 128 rows x 256 B, resident) and released to the
 //     MMA issuer on the A barrier; per unit all 128 accumulator columns are loaded, the buffer is released, and the
 //     blocked top-2 test of variants 2/3 runs on the registers (16 columns at a time, exact because the columns of a
-//     unit are rows in increasing order and the test is strict).
+//     unit are rows in increasing order and the test is strict).  K1b loads the columns packed two per register and
+//     runs the blocked test only on a unit whose minimum passes the bound (Scan::PACKED).
 // A segment switch drains the pipeline once: the readout finishes the segment's last unit (so no MMA reads A any
 // more), writes its partials, rewrites A and arrives on the A barrier.
 // A stage is released only after its reads have completed: a packed stage after the expander has stored its values
@@ -143,6 +144,52 @@ __device__ __forceinline__ void tmem_wait_ld(int (&v)[32]) {
                    "+r"(v[24]), "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]), "+r"(v[29]), "+r"(v[30]), "+r"(v[31])
                  :: "memory");
 }
+// 128 consecutive accumulator columns of this warp's 32 lanes, two per register (.pack::16b keeps the low 16 bits of
+// each column: column 2i in bits 0-15 of v[i], column 2i + 1 in bits 16-31; .x64 counts the registers).  One
+// instruction, so that no use of the first columns can be scheduled between two loads and serialise their round
+// trips; the registers hold the values only after tmem_wait_ld.
+__device__ __forceinline__ void tmem_ld128p(uint32_t taddr, uint32_t (&v)[64]) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x64.pack::16b.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, "
+                 "%13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32, %33, "
+                 "%34, %35, %36, %37, %38, %39, %40, %41, %42, %43, %44, %45, %46, %47, %48, %49, %50, %51, %52, %53, %54, "
+                 "%55, %56, %57, %58, %59, %60, %61, %62, %63}, [%64];"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
+                   "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
+                   "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31]),
+                   "=r"(v[32]), "=r"(v[33]), "=r"(v[34]), "=r"(v[35]), "=r"(v[36]), "=r"(v[37]), "=r"(v[38]), "=r"(v[39]),
+                   "=r"(v[40]), "=r"(v[41]), "=r"(v[42]), "=r"(v[43]), "=r"(v[44]), "=r"(v[45]), "=r"(v[46]), "=r"(v[47]),
+                   "=r"(v[48]), "=r"(v[49]), "=r"(v[50]), "=r"(v[51]), "=r"(v[52]), "=r"(v[53]), "=r"(v[54]), "=r"(v[55]),
+                   "=r"(v[56]), "=r"(v[57]), "=r"(v[58]), "=r"(v[59]), "=r"(v[60]), "=r"(v[61]), "=r"(v[62]), "=r"(v[63])
+                 : "r"(taddr));
+}
+__device__ __forceinline__ void tmem_wait_ld(uint32_t (&v)[64]) {
+    asm volatile("tcgen05.wait::ld.sync.aligned;"
+                 : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]),
+                   "+r"(v[8]), "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15]),
+                   "+r"(v[16]), "+r"(v[17]), "+r"(v[18]), "+r"(v[19]), "+r"(v[20]), "+r"(v[21]), "+r"(v[22]), "+r"(v[23]),
+                   "+r"(v[24]), "+r"(v[25]), "+r"(v[26]), "+r"(v[27]), "+r"(v[28]), "+r"(v[29]), "+r"(v[30]), "+r"(v[31]),
+                   "+r"(v[32]), "+r"(v[33]), "+r"(v[34]), "+r"(v[35]), "+r"(v[36]), "+r"(v[37]), "+r"(v[38]), "+r"(v[39]),
+                   "+r"(v[40]), "+r"(v[41]), "+r"(v[42]), "+r"(v[43]), "+r"(v[44]), "+r"(v[45]), "+r"(v[46]), "+r"(v[47]),
+                   "+r"(v[48]), "+r"(v[49]), "+r"(v[50]), "+r"(v[51]), "+r"(v[52]), "+r"(v[53]), "+r"(v[54]), "+r"(v[55]),
+                   "+r"(v[56]), "+r"(v[57]), "+r"(v[58]), "+r"(v[59]), "+r"(v[60]), "+r"(v[61]), "+r"(v[62]), "+r"(v[63])
+                 :: "memory");
+}
+// the two signed 16-bit halves of a packed register
+__device__ __forceinline__ int s16_lo(uint32_t x) { return static_cast<int16_t>(x & 0xFFFFu); }
+__device__ __forceinline__ int s16_hi(uint32_t x) { return static_cast<int>(x) >> 16; }
+// Signed 16x2 min of v[0 .. N - 1] as a tree of three-input mins: depth log3 N, so each level's mins issue back to back.
+template <int N>
+__device__ __forceinline__ uint32_t vmin_s16x2(const uint32_t *v) {
+    if constexpr (N == 1) {
+        return v[0];
+    } else if constexpr (N == 2) {
+        return __vmins2(v[0], v[1]);
+    } else {
+        constexpr int A = (N + 2) / 3, B = (N - A + 1) / 2;
+        return __vimin3_s16x2(vmin_s16x2<A>(v), vmin_s16x2<B>(v + A), vmin_s16x2<N - A - B>(v + A + B));
+    }
+}
 
 // Bits 4k .. 4k + 3 of w as four 0/1 bytes (byte j = bit 4k + j).
 __device__ __forceinline__ uint32_t nibble_bytes(uint32_t w, int k) { return (((w >> (4 * k)) & 0xFu) * 0x00204081u) & 0x01010101u; }
@@ -215,7 +262,10 @@ struct UmmaCols {
 //   void begin_segment(const UmmaSeg &s)              readout, after A is written
 //   UmmaCols begin_unit(const UmmaSeg &s, int i, int &thr)  unit s.u0 + i, its accumulators ready; may lower thr
 //   int threshold(unsigned long long B1)              the insert bound after an insert into (B0, B1)
-//   void loaded(int (&v)[2][32], int half, uint32_t k)  accumulator columns 64 half .. + 63 of buffer k, unmasked
+//   static constexpr bool PACKED                      the readout's form: true, all 128 columns as 16-bit halves in one
+//                                                     load and one whole-unit test; false, two halves of 64 exact
+//                                                     32-bit columns, each passed to `loaded` before the blocked test
+//   void loaded(int (&v)[2][32], int half, uint32_t k)  (PACKED false) accumulator columns 64 half .. + 63 of buffer k, unmasked
 //   void end_unit(const UmmaSeg &s, int i, uint32_t k, int rows, unsigned long long &B0, unsigned long long &B1, int &thr)
 //   void end_segment(const UmmaSeg &s, unsigned long long B0, unsigned long long B1)
 template <class Scan>
@@ -409,44 +459,82 @@ __device__ __forceinline__ void umma_pipeline(Scan &sc, const uint4 *queries, in
                 wait(AFULL + 8 * k, (c >> 1) & 1u);
                 tc_fence_after();
                 const UmmaCols u = sc.begin_unit(sg, i, thr);
-                // two halves of 64 columns (128 live values would spill); the buffer is released for unit c + 2 as soon
-                // as the second half is in registers
+                if constexpr (Scan::PACKED) {
+                    // All 128 columns in one load of 64 registers, 16 bits per column (every value is a dot in
+                    // [-256, 256]); the buffer is released for unit c + 2 before any test.  Every min is signed 16x2.
+                    uint32_t p[KNN_UMMA_ROWS / 2];
+                    tmem_ld128p(tlane + k * 256, p);
+                    tmem_wait_ld(p);
+                    tc_fence_before();
+                    mbar_arrive(AEMPTY + 8 * k);
+                    // One test for the whole unit; only a unit that can insert takes the blocked test, exact as in
+                    // the unpacked form.  In a short unit the blocks that reach past u.rows take their minimum with
+                    // those columns as 0x7FFF per 16-bit half (never below any bound), and inserts skip them by column.
+                    const uint32_t um = vmin_s16x2<KNN_UMMA_ROWS / 2>(p);
+                    if (qn + min(s16_lo(um), s16_hi(um)) < thr) {
 #pragma unroll
-                for (int half = 0; half < 2; ++half) {
-                    int v[2][32];
-                    tmem_ld32(tlane + k * 256 + static_cast<uint32_t>(64 * half), v[0]);
-                    tmem_ld32(tlane + k * 256 + static_cast<uint32_t>(64 * half + 32), v[1]);
-                    tmem_wait_ld(v[0]);
-                    tmem_wait_ld(v[1]);
-                    if (half == 1) {
-                        tc_fence_before();
-                        mbar_arrive(AEMPTY + 8 * k);
-                    }
-                    sc.loaded(v, half, k);
-                    if (u.rows < KNN_UMMA_ROWS) {
+                        for (int h = 0; h < KNN_UMMA_ROWS / 2; h += KNN_UMMA_BLOCK / 2) {
+                            const uint32_t *b = p + h;
+                            uint32_t bm = vmin_s16x2<KNN_UMMA_BLOCK / 2>(b);
+                            if (2 * h + KNN_UMMA_BLOCK > u.rows) {
+                                bm = 0x7FFF7FFFu;
 #pragma unroll
-                        for (int q = 0; q < 2; ++q)
-#pragma unroll
-                            for (int jj = 0; jj < 32; ++jj)
-                                if (64 * half + 32 * q + jj >= u.rows) v[q][jj] = 0x3FFFFFFF; // rows past the unit: never below any bound
-                    }
-#pragma unroll
-                    for (int q = 0; q < 2; ++q)
-#pragma unroll
-                        for (int h = 0; h < 32; h += KNN_UMMA_BLOCK) {
-                            int m = v[q][h];
-#pragma unroll
-                            for (int jj = 1; jj + 1 < KNN_UMMA_BLOCK; jj += 2) m = __vimin3_s32(m, v[q][h + jj], v[q][h + jj + 1]);
-                            m = min(m, v[q][h + KNN_UMMA_BLOCK - 1]);
-                            if (qn + m < thr) {
+                                for (int jj = 0; jj < KNN_UMMA_BLOCK / 2; ++jj) {
+                                    const int col = 2 * (h + jj);
+                                    bm = __vmins2(bm, col >= u.rows ? 0x7FFF7FFFu : col + 1 >= u.rows ? (b[jj] & 0xFFFFu) | 0x7FFF0000u : b[jj]);
+                                }
+                            }
+                            if (qn + min(s16_lo(bm), s16_hi(bm)) < thr) {
 #pragma unroll
                                 for (int jj = 0; jj < KNN_UMMA_BLOCK; ++jj) {
-                                    const int col = 64 * half + 32 * q + h + jj;
-                                    if (col < u.rows) top2_insert(B0, B1, make_key64(static_cast<uint32_t>(qn + v[q][h + jj]), u.key0 + col));
+                                    const int col = 2 * h + jj;
+                                    const int v = (jj & 1) ? s16_hi(b[jj >> 1]) : s16_lo(b[jj >> 1]);
+                                    if (col < u.rows) top2_insert(B0, B1, make_key64(static_cast<uint32_t>(qn + v), u.key0 + col));
                                 }
                                 thr = sc.threshold(B1);
                             }
                         }
+                    }
+                } else {
+                    // two halves of 64 columns (128 live values would spill); the buffer is released for unit c + 2 as soon
+                    // as the second half is in registers
+#pragma unroll
+                    for (int half = 0; half < 2; ++half) {
+                        int v[2][32];
+                        tmem_ld32(tlane + k * 256 + static_cast<uint32_t>(64 * half), v[0]);
+                        tmem_ld32(tlane + k * 256 + static_cast<uint32_t>(64 * half + 32), v[1]);
+                        tmem_wait_ld(v[0]);
+                        tmem_wait_ld(v[1]);
+                        if (half == 1) {
+                            tc_fence_before();
+                            mbar_arrive(AEMPTY + 8 * k);
+                        }
+                        sc.loaded(v, half, k);
+                        if (u.rows < KNN_UMMA_ROWS) {
+#pragma unroll
+                            for (int q = 0; q < 2; ++q)
+#pragma unroll
+                                for (int jj = 0; jj < 32; ++jj)
+                                    if (64 * half + 32 * q + jj >= u.rows) v[q][jj] = 0x3FFFFFFF; // rows past the unit: never below any bound
+                        }
+#pragma unroll
+                        for (int q = 0; q < 2; ++q)
+#pragma unroll
+                            for (int h = 0; h < 32; h += KNN_UMMA_BLOCK) {
+                                int m = v[q][h];
+#pragma unroll
+                                for (int jj = 1; jj + 1 < KNN_UMMA_BLOCK; jj += 2) m = __vimin3_s32(m, v[q][h + jj], v[q][h + jj + 1]);
+                                m = min(m, v[q][h + KNN_UMMA_BLOCK - 1]);
+                                if (qn + m < thr) {
+#pragma unroll
+                                    for (int jj = 0; jj < KNN_UMMA_BLOCK; ++jj) {
+                                        const int col = 64 * half + 32 * q + h + jj;
+                                        if (col < u.rows) top2_insert(B0, B1, make_key64(static_cast<uint32_t>(qn + v[q][h + jj]), u.key0 + col));
+                                    }
+                                    thr = sc.threshold(B1);
+                                }
+                            }
+                    }
                 }
                 sc.end_unit(sg, i, k, u.rows, B0, B1, thr);
 #ifdef PLM_UMMA_STAMPS
@@ -471,10 +559,12 @@ __device__ __forceinline__ void umma_pipeline(Scan &sc, const uint4 *queries, in
 // knn2_umma_kernel's units and readout: rows of one task, keys idx_base + row, the shared bound gthr, one partial slot
 // per segment.
 struct KnnScan {
+    static constexpr bool PACKED = true;
     KnnTask t;
     // per segment
     int slot, gcap;
     uint32_t *gthr;
+    uint32_t gnext; // *gthr as read one unit ahead of its use
 
     __device__ __forceinline__ int rows_of(long long u) const { return static_cast<int>(min(static_cast<long long>(KNN_UMMA_ROWS), t.n2 - u * KNN_UMMA_ROWS)); }
     __device__ __forceinline__ const uint4 *unit_src(long long u, int &rows) const {
@@ -485,12 +575,17 @@ struct KnnScan {
         slot = umma_slot(static_cast<long long>(s.g) * t.n_units, t.n1, t.n_units);
         gthr = (t.gthr && s.valid) ? t.gthr + s.qi : nullptr;
         gcap = 1023;
+        if (gthr) gnext = *reinterpret_cast<volatile uint32_t *>(gthr);
     }
     __device__ __forceinline__ UmmaCols begin_unit(const UmmaSeg &s, int i, int &thr) {
-        if (gthr) { // once per unit: the bound the other CTAs have reached (rows AT the bound stay in)
-            const uint32_t gv = *reinterpret_cast<volatile uint32_t *>(gthr);
-            gcap = static_cast<int>(min(gv, 1022u)) + 1;
+        // Once per unit: the bound the other CTAs have reached (rows AT the bound stay in), read one unit ahead so that
+        // no unit waits an L2 round trip for it.  This is exact: gthr only decreases (atomicMin), so the value read a
+        // unit earlier is >= the current one, and a larger bound only lets more rows into the insert path, whose test
+        // and top2_insert are exact.  Unit 0 of a segment uses the value read at segment start.
+        if (gthr) {
+            gcap = static_cast<int>(min(gnext, 1022u)) + 1;
             thr = min(thr, gcap);
+            gnext = *reinterpret_cast<volatile uint32_t *>(gthr); // for unit i + 1
         }
         // idx_base + n2 <= 2^32 (checked by the host)
         const long long u = s.u0 + i;
@@ -501,7 +596,6 @@ struct KnnScan {
         if (gthr && own < 1023) atomicMin(gthr, static_cast<uint32_t>(own));
         return min(own, gcap);
     }
-    __device__ __forceinline__ void loaded(int (&)[2][32], int, uint32_t) {}
     __device__ __forceinline__ void end_unit(const UmmaSeg &, int, uint32_t, int, unsigned long long &, unsigned long long &, int &) {}
     __device__ __forceinline__ void end_segment(const UmmaSeg &s, unsigned long long B0, unsigned long long B1) {
         if (!s.valid) return;

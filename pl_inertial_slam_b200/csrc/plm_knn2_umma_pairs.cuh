@@ -48,6 +48,7 @@ constexpr int KNN_UMMA_PAIRS_SMEM = KNN_UMMA_SMEM + KNN_UMMA_PAIRS_COLBUF;
 
 template <bool BOTH>
 struct PairsScan {
+    static constexpr bool PACKED = false; // direction 21 reduces the exact 32-bit values of each half (loaded)
     PairsTask t;
     // per segment
     uint32_t base21; // direction-21 key of this row: (|q| + v) << 8 | row in the group = v * 256 + base21
