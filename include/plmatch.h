@@ -731,6 +731,57 @@ typedef struct plm_localmap_params {
  * n2 * (48 + 24 is_lines) + 4 (c + 1 + k) bytes; device -> host: 4 + 9 n_sel + 4 bytes, + 4 with the grid count. */
 int plm_localmap_match_kf(plm_localmap *lm, const plm_map_view *v, const plm_localmap_kf *kf, const plm_localmap_params *p,
                           int32_t *sel, int32_t *m12, uint8_t *ok, int *n_sel, int *count);
+/* One keyframe's raw features, both kinds, as the reference holds them: points (kp: n_p x 2 float pixels,
+ * cv::KeyPoint::pt; pdesc: n_p x 32 bytes `pstep` apart; pl: n_p x 2 doubles for the gate) and segments (segs: n_l x 4
+ * float pixels sx, sy, ex, ey; ldesc; le: n_l x 3 doubles for the gate), and the shape of the grid.  Either kind may have
+ * no rows. */
+typedef struct plm_localmap_kf_raw {
+    const float *kp;
+    const uint8_t *pdesc;
+    size_t pstep;
+    const double *pl;
+    const float *segs;
+    const uint8_t *ldesc;
+    size_t lstep;
+    const double *le;
+    int32_t n_p, n_l, grid_rows, grid_cols;
+} plm_localmap_kf_raw;
+/* Outputs of one kind, as plm_localmap_match_kf writes them: sel / m12 / ok need room for plm_localmap_size entries. */
+typedef struct plm_localmap_out {
+    int32_t *sel, *m12;
+    uint8_t *ok;
+    int32_t n_sel, count;
+} plm_localmap_out;
+/* p: points, l: segments; h2d_bytes / d2h_bytes / syncs: what the call copied and how often it synchronised. */
+typedef struct plm_localmap_pl_out {
+    plm_localmap_out p, l;
+    int64_t h2d_bytes, d2h_bytes;
+    int32_t syncs, pad_;
+} plm_localmap_pl_out;
+/* The map half of MapHandler::lookForCommonMatches for one keyframe (matchMap2KFPoints, then matchMap2KFLines,
+ * mapHandler.cpp:865-871) in one call, from the keyframe's raw features.  The grids are built on the device: points go to
+ * cell (trunc(x * inv_width), trunc(y * inv_height)) of the view (off-grid points to no cell), segments to every cell of
+ * getLineCoords over the scaled endpoints, with their unit directions; items ascending inside a cell -- the host's
+ * GridStructure exactly.  Results equal two plm_localmap_match_kf calls bit for bit, given the host-built grids
+ * (grid.csr_from_points over kp * inv_width / height, drivers.line_grid) and the same pl / le; pp / pl are the two kinds'
+ * params.  Either store may be NULL (that kind is skipped, its out entries are left alone apart from n_sel = count = 0);
+ * both must be on the same context.  Every check is made on the host before any device work (PLM_E_INVALID for stores on
+ * different contexts, a store of the wrong kind, null pointers or segment endpoints more than 2^20 cells off the grid;
+ * PLM_E_GRID / PLM_E_UNSUPPORTED for grids of no cell or more than 8192 cells); a failed call changes neither store.
+ * Cost, whatever the number of landmarks (kinds whose store is NULL or empty count n = 0 and n_sel = 0):
+ *   host -> device: one copy of exactly the raw keyframe side, 56 n_p + 72 n_l bytes; no grid crosses PCIe;
+ *   device -> host: 8 bytes (both n_sel), + 8 (both grid counts, when a fallback is possible), + 9 (n_sel_p + n_sel_l)
+ *   + 8 (sel | m12 | count | ok of both kinds, one copy); with both n_sel 0 the call ends after the first 8 bytes;
+ *   synchronisations: at most 3 for the whole keyframe -- both n_sel, both grid counts (only when fast_matching and
+ *   n_sel > min_matches for a kind) and the end (besides the wait for the previous update's copy out of the same pinned
+ *   block that every call of a store makes);
+ *   launches: 1 (both grids, when some kind has landmarks, features and fast_matching) + L_p + L_l, where L_k is what
+ *   plm_localmap_match_kf launches for that kind: 3 (selection) + with n_sel > 0 and n2 > 0: 1 (gather) + matchGrid
+ *   (1; 4 with best_lr) + the brute-force fallback when it runs (knn2 + accept; twice and a cross check with best_lr)
+ *   + 1 (gate); and one device -> device copy of sel of the segments.
+ * The output cost goes to each store's h2d / d2h counters by kind (all of it to the one store when one kind runs). */
+int plm_localmap_match_kf_pl(plm_localmap *points, plm_localmap *lines, const plm_map_view *v, const plm_localmap_kf_raw *kf,
+                             const plm_localmap_params *pp, const plm_localmap_params *pl, plm_localmap_pl_out *out);
 /* Reads n slots back: X (n x 3 or 6), med_desc (n x 32 bytes), med_dir (n x 3), n_obs (observations per slot); each may
  * be NULL.  One device -> host copy and one synchronisation. */
 int plm_localmap_read(plm_localmap *lm, int n, const int32_t *idx, double *X, uint8_t *med_desc, double *med_dir, int32_t *n_obs);

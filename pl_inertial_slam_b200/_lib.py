@@ -59,6 +59,21 @@ class LocalMapParams(C.Structure):
                 ("pad_", C.c_int32)]
 
 
+class LocalMapKfRaw(C.Structure):
+    _fields_ = [("kp", vp), ("pdesc", vp), ("pstep", C.c_size_t), ("pl", vp), ("segs", vp), ("ldesc", vp),
+                ("lstep", C.c_size_t), ("le", vp), ("n_p", C.c_int32), ("n_l", C.c_int32), ("grid_rows", C.c_int32),
+                ("grid_cols", C.c_int32)]
+
+
+class LocalMapOut(C.Structure):
+    _fields_ = [("sel", vp), ("m12", vp), ("ok", vp), ("n_sel", C.c_int32), ("count", C.c_int32)]
+
+
+class LocalMapPlOut(C.Structure):
+    _fields_ = [("p", LocalMapOut), ("l", LocalMapOut), ("h2d_bytes", C.c_int64), ("d2h_bytes", C.c_int64),
+                ("syncs", C.c_int32), ("pad_", C.c_int32)]
+
+
 class PeerGroup(C.Structure):
     _fields_ = [("xchg", C.POINTER(vp)), ("gather", C.POINTER(vp)), ("rank", C.c_int32), ("world", C.c_int32),
                 ("q_cap", C.c_int32), ("pad_", C.c_int32), ("n_rows_cap", C.c_int64), ("xchg_epoch", C.c_uint32),
@@ -222,6 +237,8 @@ SIGNATURES = {
     "plm_localmap_cull": (C.c_int, [vp, C.c_int, i32p]),
     "plm_localmap_match_kf": (C.c_int, [vp, C.POINTER(MapView), C.POINTER(LocalMapKf), C.POINTER(LocalMapParams), i32p,
                                         i32p, u8p, intp, intp]),
+    "plm_localmap_match_kf_pl": (C.c_int, [vp, vp, C.POINTER(MapView), C.POINTER(LocalMapKfRaw), C.POINTER(LocalMapParams),
+                                           C.POINTER(LocalMapParams), C.POINTER(LocalMapPlOut)]),
     "plm_localmap_read": (C.c_int, [vp, C.c_int, i32p, f64p, u8p, f64p, i32p]),
     "plm_localmap_size": (C.c_int64, [vp]),
     "plm_localmap_h2d_bytes": (C.c_int64, [vp]),

@@ -19,6 +19,7 @@
 //                         kept counts the stereo stage left on the device.
 #pragma once
 #include "plm_grid.cuh"
+#include "plm_line_walk.cuh"
 #include "plm_stereo.cuh"
 
 namespace plm {
@@ -59,35 +60,6 @@ __host__ __device__ inline size_t stereo_frame_smem(const StereoCaps &c, int n_c
     b += grid_align16(static_cast<size_t>(c.cap_l) * 4);                   // m12
     if (lines) b += static_cast<size_t>(c.cap_r) * 16;                     // directions
     return b;
-}
-
-// lineIterator.cpp:34-77 + gridStructure.cpp:33-41: Bresenham from double endpoints; first cell and
-// last column come from truncation of the (possibly swapped) endpoints, error starts at dx / 2.
-// The walk is cut after max_steps cells (the host rejects frames with longer walks).
-template <class F>
-__device__ __forceinline__ void line_walk(double x1, double y1, double x2, double y2, int max_steps, F &&f) {
-    const bool steep = fabs(__dsub_rn(y2, y1)) > fabs(__dsub_rn(x2, x1));
-    if (steep) {
-        double t = x1; x1 = y1; y1 = t;
-        t = x2; x2 = y2; y2 = t;
-    }
-    if (x1 > x2) {
-        double t = x1; x1 = x2; x2 = t;
-        t = y1; y1 = y2; y2 = t;
-    }
-    const double dx = __dsub_rn(x2, x1), dy = fabs(__dsub_rn(y2, y1));
-    double error = __ddiv_rn(dx, 2.0);
-    const int ystep = (y1 < y2) ? 1 : -1;
-    int y = static_cast<int>(y1), x = static_cast<int>(x1);
-    const int max_x = static_cast<int>(x2);
-    for (int s = 0; x <= max_x && s < max_steps; ++x, ++s) {
-        f(steep ? y : x, steep ? x : y);
-        error = __dsub_rn(error, dy);
-        if (error < 0) {
-            y += ystep;
-            error = __dadd_rn(error, dx);
-        }
-    }
 }
 
 // PinholeStereoCamera::backProjection (pinholeStereoCamera.cpp:229-237).

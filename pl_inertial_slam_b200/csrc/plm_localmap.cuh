@@ -8,8 +8,12 @@
 //   med_desc[l]   32 B, med_dir[l] 3 doubles
 //   obs_start[l], obs_len[l]: the landmark's observations are rows obs_start .. obs_start + obs_len - 1 of the observation
 //                 arenas (obs_desc: 32 B per row, obs_dir: 3 doubles per row), inside a run reserved for it.
+//
+// kf_grid_kernel builds the keyframe side's grids for plm_localmap_match_kf_pl: one CTA per kind (points, segments).
 #pragma once
 #include "plm_common.cuh"
+#include "plm_grid.cuh"
+#include "plm_line_walk.cuh"
 
 namespace plm {
 
@@ -108,6 +112,136 @@ __global__ void __launch_bounds__(256) localmap_read_kernel(LmArrays m, int n, c
     }
     if (med_dir)
         for (int c = 0; c < 3; ++c) med_dir[3 * size_t(k) + c] = m.med_dir[3 * l + c];
+}
+
+// ---- keyframe grids in global memory (StVO::GridStructure as CSR, the layout of grid.py) ----------------------------
+// One kind's grid: n features (points: (x, y) float pixels; segments: (sx, sy, ex, ey)), n <= KF_GRID_MAX_FEATS.
+// cell_start: n_cells + 1 entries, cell_items: the items, unsorted: the same capacity (the fill before the in-cell sort),
+// big: n_cells entries of scratch, dirs: n x 2 unit directions (segments only).
+struct KfGridJob {
+    const float *geo;
+    int32_t *cell_start, *cell_items, *unsorted, *big;
+    double *dirs;
+    int32_t n, is_lines;
+};
+struct KfGridArgs {
+    KfGridJob job[2];
+    double inv_w, inv_h;  // of the map view: GRID_COLS / image width, GRID_ROWS / image height
+    int32_t grid_rows, grid_cols;
+};
+constexpr int KF_GRID_THREADS = 1024;
+constexpr int KF_GRID_MAX_FEATS = 32 * KF_GRID_THREADS; // one bit per feature, one bitmap word per thread
+constexpr int KF_GRID_MAX_CELLS = 8192;                 // cell counters in shared memory
+constexpr int KF_GRID_SMALL_CELL = 32;                  // larger cells are sorted through the bitmap
+
+// Exclusive sum of one value per thread over the CTA.  s_part needs blockDim.x / 32 ints.
+__device__ __forceinline__ int block_exclusive_sum(int v, int32_t *s_part) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl = v;
+#pragma unroll
+    for (int s = 1; s < 32; s <<= 1) {
+        const int t = __shfl_up_sync(0xFFFFFFFFu, incl, s);
+        if (lane >= s) incl += t;
+    }
+    if (lane == 31) s_part[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        int w = (lane < int(blockDim.x >> 5)) ? s_part[lane] : 0;
+#pragma unroll
+        for (int s = 1; s < 32; s <<= 1) {
+            const int t = __shfl_up_sync(0xFFFFFFFFu, w, s);
+            if (lane >= s) w += t;
+        }
+        if (lane < int(blockDim.x >> 5)) s_part[lane] = w;
+    }
+    __syncthreads();
+    const int r = incl - v + (warp ? s_part[warp - 1] : 0);
+    __syncthreads();
+    return r;
+}
+
+// The grid fill of stereoFrame.cpp:146-150 (points: grid.at(px * inv_width, py * inv_height), a double product truncated
+// toward zero, off-grid points go to the sink) and :336-349 (segments: every cell of getLineCoords over the scaled
+// endpoints, plus the direction (ex - sx, ey - sy) -- a float subtraction, then the double product -- normalised as
+// matching.h:43-48 does).  The CSR is the host's exactly, items in ascending feature index inside a cell (the
+// list::push_back order): a counting sort fills each cell in arbitrary order, then every cell is sorted -- small cells
+// by one thread, larger ones by the whole CTA through a bitmap of the features.
+__global__ void __launch_bounds__(KF_GRID_THREADS) kf_grid_kernel(const KfGridArgs a) {
+    extern __shared__ int32_t s_cs[]; // n_cells + 1
+    __shared__ uint32_t s_bits[KF_GRID_MAX_FEATS / 32];
+    __shared__ int32_t s_part[KF_GRID_THREADS / 32];
+    __shared__ int s_nbig;
+    const KfGridJob J = blockIdx.x ? a.job[1] : a.job[0];
+    if (J.n <= 0) return;
+    const int tid = threadIdx.x, rows = a.grid_rows, cols = a.grid_cols, n_cells = rows * cols;
+    const double inv_w = a.inv_w, inv_h = a.inv_h;
+    for (int i = tid; i <= n_cells; i += KF_GRID_THREADS) s_cs[i] = 0;
+    if (tid == 0) s_nbig = 0;
+    __syncthreads();
+    auto cells = [&](int j, auto &&f) {
+        if (!J.is_lines) {
+            const float2 k = reinterpret_cast<const float2 *>(J.geo)[j];
+            // compared as doubles: NaN and values past the int range are off the grid, as in grid.py
+            const double x = trunc(__dmul_rn(static_cast<double>(k.x), inv_w));
+            const double y = trunc(__dmul_rn(static_cast<double>(k.y), inv_h));
+            if (x >= 0.0 && x < cols && y >= 0.0 && y < rows) f(static_cast<int>(x) * rows + static_cast<int>(y));
+        } else {
+            // the host bounds the scaled endpoints (|v| <= 2^20), so the whole walk runs, as the reference's does
+            const float4 k = reinterpret_cast<const float4 *>(J.geo)[j];
+            line_walk(__dmul_rn(static_cast<double>(k.x), inv_w), __dmul_rn(static_cast<double>(k.y), inv_h),
+                      __dmul_rn(static_cast<double>(k.z), inv_w), __dmul_rn(static_cast<double>(k.w), inv_h), INT_MAX,
+                      [&](int x, int y) {
+                          if (x >= 0 && x < cols && y >= 0 && y < rows) f(x * rows + y);
+                      });
+        }
+    };
+    for (int j = tid; j < J.n; j += KF_GRID_THREADS) {
+        cells(j, [&](int c) { atomicAdd(&s_cs[c], 1); });
+        if (J.is_lines) {
+            const float4 k = reinterpret_cast<const float4 *>(J.geo)[j];
+            const double vx = __dmul_rn(static_cast<double>(__fsub_rn(k.z, k.x)), inv_w);
+            const double vy = __dmul_rn(static_cast<double>(__fsub_rn(k.w, k.y)), inv_h);
+            const double mag = __dsqrt_rn(__dadd_rn(__dmul_rn(vx, vx), __dmul_rn(vy, vy)));
+            J.dirs[2 * j] = __ddiv_rn(vx, mag);
+            J.dirs[2 * j + 1] = __ddiv_rn(vy, mag);
+        }
+    }
+    __syncthreads();
+    block_inclusive_scan(s_cs, n_cells, s_part); // cell ends
+    if (tid == 0) s_cs[n_cells] = s_cs[n_cells - 1];
+    __syncthreads();
+    for (int j = tid; j < J.n; j += KF_GRID_THREADS)
+        cells(j, [&](int c) { J.unsorted[atomicSub(&s_cs[c], 1) - 1] = j; });
+    __syncthreads(); // s_cs[c] = start of cell c
+    for (int i = tid; i <= n_cells; i += KF_GRID_THREADS) J.cell_start[i] = s_cs[i];
+    for (int c = tid; c < n_cells; c += KF_GRID_THREADS) {
+        const int s = s_cs[c], m = s_cs[c + 1] - s;
+        if (m > KF_GRID_SMALL_CELL) {
+            J.big[atomicAdd(&s_nbig, 1)] = c;
+            continue;
+        }
+        for (int k = 0; k < m; ++k) { // insertion sort
+            const int32_t v = J.unsorted[s + k];
+            int p = k;
+            for (; p > 0 && J.cell_items[s + p - 1] > v; --p) J.cell_items[s + p] = J.cell_items[s + p - 1];
+            J.cell_items[s + p] = v;
+        }
+    }
+    __syncthreads();
+    const int n_big = s_nbig, words = (J.n + 31) / 32;
+    for (int b = 0; b < n_big; ++b) {
+        const int c = J.big[b], s = s_cs[c], m = s_cs[c + 1] - s;
+        if (tid < words) s_bits[tid] = 0;
+        __syncthreads();
+        for (int k = tid; k < m; k += KF_GRID_THREADS) {
+            const int32_t v = J.unsorted[s + k];
+            atomicOr(&s_bits[v >> 5], 1u << (v & 31));
+        }
+        __syncthreads();
+        uint32_t w = tid < words ? s_bits[tid] : 0u;
+        int p = s + block_exclusive_sum(__popc(w), s_part);
+        for (; w; w &= w - 1) J.cell_items[p++] = tid * 32 + (__ffs(w) - 1);
+    }
 }
 
 } // namespace plm

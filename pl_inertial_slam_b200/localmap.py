@@ -12,6 +12,7 @@ with the map.  Results equal drivers.matchMap2KF*Full on the same landmarks bit 
     local bundle adjustment -> set_positions
     local-map bookkeeping -> set_active / cull
     matchMap2KF*          -> matchMap2KFPoints / matchMap2KFLines (one plm_localmap_match_kf call)
+    lookForCommonMatches  -> match_keyframe: both kinds of one keyframe in one call, grids built on the device
 
 One store holds one kind (points or segments), as the reference keeps map_points and map_lines apart.  A landmark's
 index is its slot: slots are handed out in insertion order and never reused.  One host thread at a time per store."""
@@ -35,6 +36,16 @@ def _p(a: np.ndarray, t):
 
 def _idx(idx) -> np.ndarray:
     return np.ascontiguousarray(np.asarray(idx, np.int64).reshape(-1), np.int32)
+
+
+def _params(nnr: float, min_matches: int, max_epip: float) -> L.LocalMapParams:
+    """The config values matchMap2KFPoints / Lines read, as plm_localmap_params."""
+    p = L.LocalMapParams()
+    p.ratio, p.line_sim_th, p.max_epip = float(M.Config.minRatio12P), float(M.Config.lineSimTh), float(max_epip)
+    p.nnr, p.ws = float(np.float32(nnr)), int(M.Config.matchingF2FWs)
+    p.best_lr, p.fast_matching = int(bool(M.Config.bestLRMatches)), int(bool(D.SlamConfig.fastMatching))
+    p.min_matches = int(min_matches)
+    return p
 
 
 class LocalMap:
@@ -136,11 +147,7 @@ class LocalMap:
             dirs2 = np.ascontiguousarray(dirs2, np.float64).reshape(-1, 2)
             kf.dirs2 = dirs2.ctypes.data
         kf.n2, kf.grid_rows, kf.grid_cols = n2, G.GRID_ROWS, G.GRID_COLS
-        p = L.LocalMapParams()
-        p.ratio, p.line_sim_th, p.max_epip = float(M.Config.minRatio12P), float(M.Config.lineSimTh), float(max_epip)
-        p.nnr, p.ws = float(np.float32(nnr)), int(M.Config.matchingF2FWs)
-        p.best_lr, p.fast_matching = int(bool(M.Config.bestLRMatches)), int(bool(D.SlamConfig.fastMatching))
-        p.min_matches = int(min_matches)
+        p = _params(nnr, min_matches, max_epip)
         cap = max(len(self), 1)
         sel, m12, ok = np.zeros(cap, np.int32), np.zeros(cap, np.int32), np.zeros(cap, np.uint8)
         n_sel, count = C.c_int(0), C.c_int(0)
@@ -182,3 +189,51 @@ class LocalMap:
             self.close()
         except Exception:
             pass
+
+
+def match_keyframe(points_map: Optional[LocalMap], lines_map: Optional[LocalMap], view: L.MapView, kp_px, pdesc, pl, ln_px,
+                   ldesc, le, grid_rows: int = G.GRID_ROWS, grid_cols: int = G.GRID_COLS) -> dict:
+    """The map half of MapHandler::lookForCommonMatches for one keyframe (matchMap2KFPoints, then matchMap2KFLines) in one
+    plm_localmap_match_kf_pl call, from the keyframe's raw features: the grids are built on the device.
+
+    kp_px: n_p x 2 float32 pixel keypoints, pdesc: n_p x 32, pl: n_p x 2 for the gate (None = kp_px); ln_px: n_l x 4
+    float32 pixel segments, ldesc: n_l x 32, le: n_l x 3.  Either map may be None (that kind is skipped).  Returns
+    dict(points=..., lines=..., cost=...): per kind the dict of LocalMap.matchMap2KFPoints / Lines (sel, m12, ok,
+    matches), None for a skipped kind; cost = dict(h2d_bytes, d2h_bytes, syncs) of the call."""
+    if points_map is not None and points_map.is_lines:
+        raise ValueError("points_map holds segments")
+    if lines_map is not None and not lines_map.is_lines:
+        raise ValueError("lines_map holds points")
+    lib = L.load()
+    kp = np.ascontiguousarray(np.asarray(kp_px if kp_px is not None else np.zeros((0, 2)), np.float32).reshape(-1, 2))
+    ln = np.ascontiguousarray(np.asarray(ln_px if ln_px is not None else np.zeros((0, 4)), np.float32).reshape(-1, 4))
+    pd, _, n_p, pstep = L.desc_args(np.asarray(pdesc if pdesc is not None else np.zeros((0, 32)), np.uint8).reshape(-1, 32))
+    ld, _, n_l, lstep = L.desc_args(np.asarray(ldesc if ldesc is not None else np.zeros((0, 32)), np.uint8).reshape(-1, 32))
+    plv = np.ascontiguousarray(kp if pl is None else np.asarray(pl), np.float64).reshape(-1, 2)
+    lev = np.ascontiguousarray(np.asarray(le if le is not None else np.zeros((0, 3)), np.float64)).reshape(-1, 3)
+    if len(kp) != n_p or len(plv) != n_p:
+        raise ValueError("kp_px / pl need one row per point descriptor")
+    if len(ln) != n_l or len(lev) != n_l:
+        raise ValueError("ln_px / le need one row per segment descriptor")
+    kf = L.LocalMapKfRaw()
+    kf.kp, kf.pdesc, kf.pstep, kf.pl = kp.ctypes.data, pd.ctypes.data, pstep.value, plv.ctypes.data
+    kf.segs, kf.ldesc, kf.lstep, kf.le = ln.ctypes.data, ld.ctypes.data, lstep.value, lev.ctypes.data
+    kf.n_p, kf.n_l, kf.grid_rows, kf.grid_cols = n_p, n_l, int(grid_rows), int(grid_cols)
+    pp = _params(M.Config.minRatio12P, D.SlamConfig.minPointMatches, D.SlamConfig.maxKFEpipP)
+    pln = _params(M.Config.minRatio12L, D.SlamConfig.minLineMatches, D.SlamConfig.maxKFEpipL)
+    out = L.LocalMapPlOut()
+    bufs = []
+    for m, o in ((points_map, out.p), (lines_map, out.l)):
+        cap = max(len(m), 1) if m is not None else 1
+        b = (np.zeros(cap, np.int32), np.zeros(cap, np.int32), np.zeros(cap, np.uint8))
+        o.sel, o.m12, o.ok = b[0].ctypes.data, b[1].ctypes.data, b[2].ctypes.data
+        bufs.append(b)
+    L.check(lib.plm_localmap_match_kf_pl(points_map._h if points_map is not None else None,
+                                         lines_map._h if lines_map is not None else None, C.byref(view), C.byref(kf),
+                                         C.byref(pp), C.byref(pln), C.byref(out)), "plm_localmap_match_kf_pl")
+    res = {}
+    for name, m, o, b in (("points", points_map, out.p, bufs[0]), ("lines", lines_map, out.l, bufs[1])):
+        k = o.n_sel
+        res[name] = None if m is None else dict(sel=b[0][:k].copy(), m12=b[1][:k].copy(), ok=b[2][:k].copy(), matches=o.count)
+    res["cost"] = dict(h2d_bytes=out.h2d_bytes, d2h_bytes=out.d2h_bytes, syncs=out.syncs)
+    return res
